@@ -23,11 +23,14 @@ that block.  Multi-GPU: the recording is time-sharded, every rank owns a contigu
              (sa_spectrogram_file), and as a display canvas (only W x H x 4 bytes come back)
 
 --impl reference times that CPU port alone (the reference itself is Java; no JVM in the image).
+--dump-outputs DIR writes a fixed, seeded sample of rows of the dB image of the last timed step (rank 0) as .npy files;
+the recording is generated from fixed seeds, so two builds run with the same arguments can be compared row for row.
 """
 import argparse
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -213,6 +216,25 @@ def timed_ms(torch, fn, steps, warmup=3):
     return t[len(t) // 2]
 
 
+DUMP_ROWS = 8192        # 8192 rows x 1024 bins x 4 B = 32 MiB
+
+
+def dump_outputs(out_dir, d_out):
+    """Writes what the timed step returns to its caller -- the [frames, NFFT] float32 dB image -- as a fixed sample: the
+    first and last rows plus rows drawn with a fixed seed, so that two builds can be compared row for row."""
+    import numpy as np
+    import torch
+    frames = d_out.shape[0]
+    rows = np.arange(frames)
+    if frames > DUMP_ROWS:
+        inner = np.random.default_rng(0).choice(rows[1:-1], size=DUMP_ROWS - 2, replace=False)
+        rows = np.sort(np.concatenate([[0], inner, [frames - 1]]))
+    os.makedirs(out_dir, exist_ok=True)
+    img = d_out.index_select(0, torch.from_numpy(rows).to(d_out.device)).cpu().numpy()
+    np.save(os.path.join(out_dir, "spectrogram_db_rows.npy"), img)
+    np.save(os.path.join(out_dir, "spectrogram_row_index.npy"), rows.astype(np.float64))
+
+
 def other_configs(eng, steps, scale):
     """BASELINE.json configs[1..4] device-resident on one GPU, each with its own roofline record (algorithmic
     bytes of SURVEY.md 8d / median CUDA-event time / measured HBM peak).  Inputs + outputs of every case are far
@@ -261,7 +283,11 @@ def main():
     ap.add_argument("--configs-scale", type=float, default=1.0, help="shrinks the sample counts of the other configurations")
     ap.add_argument("--sustained-steps", type=int, default=400,
                     help="extra back-to-back steps timed as one region to show the power-capped rate (0: skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed sample of rank 0's dB image from the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -331,6 +357,8 @@ def main():
     sampler.join()
     launches = eng.kernel_launches - launches0
     kernel_name = eng.last_kernel              # what the engine actually launched (sa_last_kernel_name), not a literal
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, d_out)
     per_step = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
     ms = max_over_ranks(ev[0].elapsed_time(ev[args.steps]) / args.steps)
     samples_per_step_local = frames * HOP
@@ -471,7 +499,9 @@ def main():
         # the app's own input: the .sigmf-data file.  (a) file-backed mmap in, pageable array out -- the
         # MappedByteBuffer of SigMfHelper.java:78-84, which cannot be page-locked; (b) the engine reads the file itself
         tmpdir = "/dev/shm" if os.path.isdir("/dev/shm") else "/tmp"
-        path = os.path.join(tmpdir, "sa_bench_rank%d.sigmf-data" % rank)
+        # a unique name: another user's file of the same name in the shared directory must not break this leg
+        fd, path = tempfile.mkstemp(prefix="sa_bench_rank%d_" % rank, suffix=".sigmf-data", dir=tmpdir)
+        os.close(fd)
         try:
             st = os.statvfs(tmpdir)
             if st.f_bavail * st.f_frsize < 2 * world * n_local * 8:

@@ -37,6 +37,34 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert r.returncode == 0 and not [l for l in r.stdout.splitlines() if l.startswith("{")]
 
 
+def test_dump_outputs_is_a_fixed_bounded_sample(tmp_path):
+    """--dump-outputs: the same rows (first, last and a seeded sample) on every run, each row exactly as computed, and at
+    most 64 MiB in all; a small image is written whole."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    frames = 100003
+    img = torch.arange(frames, dtype=torch.float32)[:, None] + torch.arange(bench.NFFT, dtype=torch.float32) / bench.NFFT
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), img)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == ["spectrogram_db_rows.npy", "spectrogram_row_index.npy"]
+    got = {f: np.load(tmp_path / "a" / f) for f in files}
+    assert all(np.array_equal(v, np.load(tmp_path / "b" / f)) for f, v in got.items())
+    rows, idx = got["spectrogram_db_rows.npy"], got["spectrogram_row_index.npy"]
+    assert rows.dtype == np.float32 and idx.dtype == np.float64 and rows.nbytes + idx.nbytes <= 64 << 20
+    assert len(np.unique(idx)) == len(idx) == bench.DUMP_ROWS and idx[0] == 0 and idx[-1] == frames - 1
+    assert np.array_equal(rows, img.numpy()[idx.astype(np.int64)])
+    bench.dump_outputs(str(tmp_path / "c"), img[:10])
+    assert np.array_equal(np.load(tmp_path / "c" / "spectrogram_db_rows.npy"), img[:10].numpy())
+
+
+def test_steps_must_be_positive():
+    r = run_bench("--steps", "0")
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_product_arm_has_no_cpu_fallback():
     import torch
     if torch.cuda.is_available():

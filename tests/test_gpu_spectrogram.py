@@ -161,7 +161,7 @@ def test_linearity_and_time_shift_properties(engine):
     assert np.abs(p / e - 1).max() < 1e-4
 
 
-def test_both_1024_kernels_against_oracle(engine):
+def test_both_1024_kernels_against_oracle(engine, tmp_path):
     """The 1024-point FP32 plan has two kernels: TMA-staged frames (16-byte aligned frame starts) and
     the LDG kernel (any alignment, or SA_NO_TMA=1).  Both are checked against the oracle; the LDG
     kernel on aligned input runs in a subprocess because the switch is read once per process."""
@@ -179,7 +179,7 @@ def test_both_1024_kernels_against_oracle(engine):
             "raw = synth.recording(1024 * 40, 'cf32_le', seed=31);"
             "np.save(sys.argv[1], e.spectrogram(raw, 'cf32_le', 1024, 70, hop=512, window='hann'))"
             % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    out = os.path.join(os.environ.get("TMPDIR", "/tmp"), "sa_no_tma.npy")
+    out = str(tmp_path / "sa_no_tma.npy")
     env = dict(os.environ, SA_NO_TMA="1")
     subprocess.run([sys.executable, "-c", code, out], check=True, env=env)
     got_ldg = np.load(out)
