@@ -614,10 +614,6 @@ void fill_load_params(LoadParams& lp, const void* base, int dtype, int big_endia
 
 static bool is_pow2(uint64_t x) { return x && !(x & (x - 1)); }
 
-// strict_reference: datatypes SpectralService.computeMagnitudes has no branch for decode to zeros (:60-63)
-static bool strict_zero(const sa_spectrogram_params& p) {
-    return p.strict_reference && (p.dtype == SA_CF64 || p.dtype == SA_DT_OTHER);
-}
 // bytes per IQ pair as the frame loop sees them: Global.getBytesPerSample (S/sigmf/Global.java:67-79), fallback 8
 uint64_t spec_bytes_per_iq(const sa_spectrogram_params& p) {
     if (p.dtype == SA_DT_OTHER) return p.strict_reference ? 8 : 0;
@@ -700,7 +696,7 @@ int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_sp
         a.cmap = p.colormap;
     }
     if (pool_mode) {
-        if (!can_pool(p, prec) || strict_zero(p)) return set_error(SA_ERR_UNSUPPORTED, "fused pooling covers the in-SM transforms only");
+        if (!can_pool(p, prec)) return set_error(SA_ERR_UNSUPPORTED, "fused pooling covers the in-SM transforms only");
         a.pool_mode = pool_mode;
         a.pool_fpc = (long long)std::max<uint64_t>(1, pool_fpc);
         a.pool_magic = a.pool_fpc > 1 ? (unsigned long long)((((unsigned __int128)1 << 64) + (unsigned __int128)(a.pool_fpc - 1)) / (unsigned __int128)a.pool_fpc) : 0ull;

@@ -26,6 +26,10 @@ bool host_ptr_is_pinned(const void* p);     // pinned / registered host memory (
 int check_spec_params(const sa_spectrogram_params* p, int* prec_out);   // validates, resolves precision
 void fill_load_params(LoadParams& lp, const void* base, int dtype, int big_endian);
 uint64_t spec_bytes_per_iq(const sa_spectrogram_params& p);   // Global.getBytesPerSample, strict_reference aware
+// strict_reference: datatypes SpectralService.computeMagnitudes has no branch for decode to zeros (:60-63)
+inline bool strict_zero(const sa_spectrogram_params& p) {
+    return p.strict_reference && (p.dtype == SA_CF64 || p.dtype == SA_DT_OTHER);
+}
 
 // Where the host pipeline takes a capture's bytes from: caller memory (pinned: DMA source as is; pageable:
 // parallel memcpy into the pinned ring) or an open file (parallel pread straight into the pinned ring).
@@ -137,10 +141,13 @@ struct Engine {
     int launch_spectrogram_large(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
                                  const SpecArgs& base, void* d_out, cudaStream_t stream, int ws);
     // pool_mode != 0: instead of rows, |X|^2 is reduced (1 max, 2 sum) over the pool_fpc frames of each canvas column into
-    // d_out = float[n_frames / pool_fpc][nfft], which the caller has zeroed (display.cu); transforms up to 16384 points
+    // d_out = float[n_frames / pool_fpc][nfft], which the caller has zeroed (display.cu); transforms up to 16384 points.
+    // A strict_zero request transforms nothing (its rows are constants): it takes the rows path, not the pooling one.
     int launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
                            void* d_out, cudaStream_t stream, int ws = 2, int pool_mode = 0, uint64_t pool_fpc = 1);
-    static bool can_pool(const sa_spectrogram_params& p, int prec) { return p.nfft <= 16384 && !(prec == SA_PREC_F64 && p.nfft > 8192); }
+    static bool can_pool(const sa_spectrogram_params& p, int prec) {
+        return p.nfft <= 16384 && !(prec == SA_PREC_F64 && p.nfft > 8192) && !strict_zero(p);
+    }
     int spectrogram_host(const HostSource& src, uint64_t iq_bytes, const sa_spectrogram_params& p, int prec, void* out);
 };
 

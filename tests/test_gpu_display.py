@@ -44,7 +44,8 @@ def test_canvas_matches_render_spectrogram(engine, cmap, dt, nfft, W, H):
 
 @pytest.mark.parametrize("reduce", ["max", "mean"])
 def test_canvas_pooling_whole_recording(engine, reduce):
-    """several frames and bins per pixel; also more columns than one 64 MiB chunk holds (chunked pipeline)."""
+    """several frames and bins per pixel, in one host chunk (test_gpu_kernel_matrix.py covers canvases of several
+    64 MiB chunks and pooled launches past one wave)."""
     fs, nfft, hop, fpc, W, H = 1.0e6, 512, 256, 5, 41, 96
     raw = synth.recording((W * fpc - 1) * hop + nfft, "ci16_le", seed=29)
     db = co.spectrogram(raw, "ci16_le", 0, nfft, hop, "hann", W * fpc)
@@ -64,6 +65,69 @@ def test_canvas_pooling_whole_recording(engine, reduce):
                                reduce=reduce, colormap="Heatmap", min_db=lo, max_db=hi)
     n = np.clip((pooled.T[::-1] - conv - lo) / (hi - lo), 0, 1)
     pixel_check(got, ref, n[..., None].repeat(4, -1), "Heatmap", max_frac=0.08)
+
+
+_STRICT_ROWS_PATH = """
+import sys
+import numpy as np
+sys.path.insert(0, sys.argv[1])
+import spectral_analyzer_b200 as sa
+e = sa.Engine(0)
+raw = np.load(sys.argv[2])
+out = {}
+for dt, bps in (("cf64_le", 16), ("ri16_le", 8)):
+    data = raw[:(9 * 3 - 1) * 1024 * bps + 1024 * bps]
+    for reduce in ("max", "mean"):
+        out[dt + reduce] = e.render_canvas(data, dt, 1024, 12, 64, 1.0e6, frames_per_column=3, reduce=reduce,
+                                           strict_reference=True, min_db=float(sys.argv[4]), max_db=float(sys.argv[5]))
+np.savez(sys.argv[3], **out)
+"""
+
+
+def test_strict_reference_pooled_canvas(engine, tmp_path):
+    """strict_reference with a datatype the reference cannot decode (cf64, SA_DT_OTHER): every readable frame is
+    -200 dB and the pooled MAX / MEAN canvas shows just that, past EOF the -150 dB fill, on the host and the device
+    path, identical to the canvas of dB rows (SA_CANVAS_FUSED=0, read once per process: a subprocess)."""
+    import subprocess
+    import sys
+    import ctypes as C
+    import torch
+    from spectral_analyzer_b200 import _capi
+    fs, nfft, W, H, fpc = 1.0e6, 1024, 12, 64, 3
+    conv = 10 * np.log10(fs / nfft) + 20 * np.log10(nfft)
+    lo, hi = float(-200.0 - conv - 10.0), float(-150.0 - conv + 10.0)
+    colour = {v: co.render_rgba(np.full((1, nfft), v), fs, lo, hi, "Grayscale")[0, 0] for v in (-200.0, -150.0)}
+    assert not np.array_equal(colour[-200.0], colour[-150.0])
+    wr = 9                                                   # the frames of columns 9..11 lie past EOF
+    raw = np.random.default_rng(3).integers(0, 256, (wr * fpc - 1) * nfft * 16 + nfft * 16, dtype=np.uint8)
+    got = {}
+    for dt in ("cf64_le", "ri16_le"):
+        bps = 16 if dt == "cf64_le" else 8                   # ri16_le: Global.getBytesPerSample's fallback
+        data = raw[:(wr * fpc - 1) * nfft * bps + nfft * bps]
+        for reduce in ("max", "mean"):
+            g = engine.render_canvas(data, dt, nfft, W, H, fs, frames_per_column=fpc, reduce=reduce,
+                                     strict_reference=True, min_db=lo, max_db=hi)
+            assert (g[:, :wr] == colour[-200.0]).all() and (g[:, wr:] == colour[-150.0]).all(), (dt, reduce)
+            got[dt + reduce] = g
+            d_iq = torch.from_numpy(data).cuda()
+            d_out = torch.empty(W * H * 4, dtype=torch.uint8, device="cuda")
+            p = engine.make_params(dt, nfft, None, "rect", 0, 0, sample_rate=fs, min_db=lo, max_db=hi,
+                                   strict_reference=True)
+            _capi.check(_capi.lib().sa_render_canvas_device(engine.handle, d_iq.data_ptr(), data.size, C.byref(p), W, H,
+                                                            fpc, _capi.REDUCE[reduce], d_out.data_ptr(),
+                                                            torch.cuda.current_stream().cuda_stream))
+            torch.cuda.synchronize()
+            assert np.array_equal(d_out.view(H, W, 4).cpu().numpy(), g), (dt, reduce)
+    np.save(tmp_path / "raw.npy", raw)
+    script = tmp_path / "rows_path.py"
+    script.write_text(_STRICT_ROWS_PATH)
+    env = dict(os.environ, SA_CANVAS_FUSED="0")
+    subprocess.run([sys.executable, str(script), os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
+                    str(tmp_path / "raw.npy"), str(tmp_path / "rows.npz"), repr(lo), repr(hi)], check=True, env=env)
+    rows = np.load(tmp_path / "rows.npz")
+    for dt in ("cf64_le", "ri16_le"):
+        for reduce in ("max", "mean"):
+            assert np.array_equal(rows[dt + reduce], got[dt + reduce]), (dt, reduce)
 
 
 def test_canvas_argument_errors(engine):

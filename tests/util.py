@@ -35,3 +35,18 @@ def check_db_parity(got, ref, mode_power=False, strong_tol=DB_OF_REL_POWER, floo
     lin_max = 10 ** (fmax / scale)
     assert (np.abs(lin_g - lin_r) <= 1e-5 * lin_max).all()
     return worst_strong, worst_above
+
+
+# Norm-wise bounds of frame_norm_error: 2x and 3x the worst E measured on white noise (tests/test_gpu_kernel_matrix.py)
+NORM_TOL_F32 = 1e-5
+NORM_TOL_F64 = 1e-12
+
+
+def frame_norm_error(got, ref):
+    """Per frame E = max_k |A_got - A_ref| / rms_k(A_ref), A = 10^(dB/20) the linear magnitude (also in power mode,
+    which writes 10 log10 |X|^2).  Unlike check_db_parity it holds EVERY bin of a full-band frame to the same
+    absolute scale, so a wrong frame, a shifted bin or a mis-scaled bin shows however weak the bin is.
+    got, ref: dB images [frames, nfft]; returns float64 [frames]."""
+    a_g = np.power(10.0, np.asarray(got, np.float64) / 20.0)
+    a_r = np.power(10.0, np.asarray(ref, np.float64) / 20.0)
+    return np.abs(a_g - a_r).max(axis=1) / np.sqrt(np.mean(a_r * a_r, axis=1))
