@@ -310,7 +310,7 @@ static int welch_launch(Engine* eng, const WelchLaunch& wl, const WelchSig* d_si
     for (uint32_t i = 1; i < n_sig && contiguous; i++) contiguous = wl.d_out[i] == wl.d_out[i - 1] + nfft;
     const size_t out_bytes = contiguous ? 0 : (((size_t)n_sig * nfft * sizeof(double) + 255) & ~(size_t)255);
     const size_t part_bytes = wk ? (size_t)n_sig * wl.nsplit * wk->slots * nfft * elem : 0;
-    const int slot = wsi ? 13 : 1;
+    const int slot = wsi ? 9 : 1;
     int rc = eng->ensure_scratch(slot, std::max<size_t>(sig_bytes + out_bytes + part_bytes, 256) + 256);      // + the task counter
     if (rc) return rc;
     char* base = (char*)eng->scratch[slot];
@@ -501,7 +501,7 @@ static int run_batch_device(Engine* eng, const void* d_iq, uint64_t n_samples, i
     const bool dual = want_psd && batches.size() > 1;
     int rc = SA_OK;
     if (want_psd) {
-        rc = eng->ensure_scratch(12, (dual ? 2 : 1) * std::max<uint64_t>(scr_total, 1) * sizeof(float2));
+        rc = eng->ensure_scratch(8, (dual ? 2 : 1) * std::max<uint64_t>(scr_total, 1) * sizeof(float2));
         if (rc) return rc;
     }
     // annotation plan (device): batch by batch, inside a batch sorted by (kernel, fast, down) so that launches group
@@ -524,7 +524,7 @@ static int run_batch_device(Engine* eng, const void* d_iq, uint64_t n_samples, i
     if (want_psd) {
         for (size_t bi = 0; bi < batches.size(); bi++) {
             const int par = dual ? (int)(bi & 1) : 0;
-            const float2* scr = (const float2*)eng->scratch[12] + (size_t)par * scr_total;
+            const float2* scr = (const float2*)eng->scratch[8] + (size_t)par * scr_total;
             std::map<uint32_t, std::vector<WelchJob>> by_n;
             for (uint32_t i = batches[bi].first; i < batches[bi].second; i++) {
                 WelchJob j;
@@ -632,7 +632,7 @@ static int run_batch_device(Engine* eng, const void* d_iq, uint64_t n_samples, i
             if (e != cudaSuccess) return cuda_fail(e, "analysis pipeline wait");
         }
         const uint32_t bn = batches[bi].second - batches[bi].first;
-        da.scratch = want_psd ? (float2*)eng->scratch[12] + (size_t)par * scr_total : nullptr;
+        da.scratch = want_psd ? (float2*)eng->scratch[8] + (size_t)par * scr_total : nullptr;
         for (uint32_t g0 = pos; g0 < pos + bn;) {
             uint32_t g1 = g0 + 1;
             while (g1 < pos + bn && key(order[g1]) == key(order[g0])) g1++;

@@ -16,12 +16,6 @@
 
 namespace sa {
 
-#ifndef SA_LARGE_DUAL_DEFAULT
-#define SA_LARGE_DUAL_DEFAULT 0
-#endif
-constexpr bool kLargeDualDefault = SA_LARGE_DUAL_DEFAULT != 0;
-constexpr uint64_t kLargeDualWsMb = 48;
-
 // ---------------- parallel host copies ----------------
 CopyPool::CopyPool(int workers) {
     for (int i = 0; i < workers; i++) threads_.emplace_back([this] { worker(); });
@@ -288,27 +282,9 @@ int Engine::mid_t1_table(int n, const void** d_tab) {
     return SA_OK;
 }
 
-// cuTensorMapEncodeTiled through the runtime's driver entry point lookup (no link against libcuda)
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFn encode_tiled_fn() {
-    static EncodeTiledFn fn = [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            p = nullptr;
-        }
-        return (EncodeTiledFn)p;
-    }();
-    return fn;
-}
-
-// Four-step path (large_fft_kernels.cuh): frames are processed in chunks whose workspace stays L2-sized.
-int Engine::launch_spectrogram_large(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
-                                     const SpecArgs& base, void* d_out, cudaStream_t stream, int ws) {
-    (void)d_iq; (void)n_samples; (void)d_out;
+// Four-step path (large_fft_kernels.cuh): frames are processed in chunks of at most 512 MiB of workspace, each chunk
+// one large_cols_kernel and one large_rows_kernel launch on the caller's stream.
+int Engine::launch_spectrogram_large(const sa_spectrogram_params& p, int prec, const SpecArgs& base, cudaStream_t stream, int ws) {
     const int dk = dtype_kind(p.dtype);
     const int win = (prec == SA_PREC_F64) ? 1 : (p.window != SA_WIN_RECT ? 1 : 0);
     const LargeKernelInfo* k = find_large_kernel(prec, (int)p.nfft, dk, win);
@@ -330,252 +306,28 @@ int Engine::launch_spectrogram_large(const void* d_iq, uint64_t n_samples, const
     if (win) { rc = window_table(p.window, (int)p.nfft, prec, &a.s.window); if (rc) return rc; }
     const size_t elem = (prec == SA_PREC_F64) ? 16 : 8;
     const uint64_t per_frame = (uint64_t)p.nfft * elem;
-    void* args[] = { &a };
-    cudaError_t e;
-    // 65536 points with 16-byte aligned frames, opt-in (SA_LARGE_ONCHIP=1): the on-chip cluster kernel (the frame stays
-    // in the distributed shared memory of an 8-CTA cluster between the column and the row step; no workspace, DRAM
-    // traffic = algorithmic bytes).  Measured on B200 it LOSES to the two-kernel path (config 5: 1.32 vs 0.785 ms; FP32:
-    // 1.04 vs 0.683 ms): one 256-thread CTA per SM leaves every phase latency-bound and the phases of a frame are
-    // serialised by two cluster barriers (per frame and CTA, FP64, cycles: column FFTs 11.3 k, barrier 2.1 k, DSMEM pull
-    // 5.3 k = 24 B/clk, barrier 5.0 k, row FFTs 7.0 k, dB + store 8.9 k; TMA wait 0.8 k, i.e. the loads ARE hidden) --
-    // the two kernels are issue-bound, not bound by the workspace round trip (DESIGN.md K6).
-    const char* onchip_env = getenv("SA_LARGE_ONCHIP");               // read per call: the tests A/B the two paths
-    const bool use_onchip = onchip_env ? atoi(onchip_env) != 0 : false;
-    const uint64_t iq_b = (uint64_t)sa_bytes_per_iq(p.dtype);
-    const bool aligned = ((uintptr_t)d_iq % 16 == 0) && ((p.start_sample * iq_b) % 16 == 0) && ((p.hop * iq_b) % 16 == 0);
-    if (k->fn_cluster && use_onchip && aligned) {
-        auto it = occupancy.find(k->fn_cluster);
-        int n_clusters = 0;
-        cudaLaunchConfig_t cfg;
-        memset(&cfg, 0, sizeof(cfg));
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = kLargeCluster; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.blockDim = dim3(k->cta_cluster);
-        cfg.dynamicSmemBytes = k->smem_cluster;
-        cfg.stream = stream;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        if (it == occupancy.end()) {
-            e = cudaFuncSetAttribute(k->fn_cluster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_cluster);
-            if (e != cudaSuccess) return cuda_fail(e, "on-chip four-step smem attribute");
-            cfg.gridDim = dim3(kLargeCluster * num_sms);
-            e = cudaOccupancyMaxActiveClusters(&n_clusters, k->fn_cluster, &cfg);
-            if (e != cudaSuccess || n_clusters < 1) { cudaGetLastError(); n_clusters = 0; }
-            occupancy[k->fn_cluster] = n_clusters;
-        } else {
-            n_clusters = it->second;
-        }
-        // tensor map [frame][n1][n2] over the readable frames, in 8-byte elements: strides hop and 256 samples
-        // (frames overlap when hop < nfft), box = 16 columns x 256 rows x 1 frame
-        const uint64_t first_end = p.start_sample + p.nfft;
-        const uint64_t n_read = n_samples >= first_end ? std::min<uint64_t>(p.n_frames, (n_samples - first_end) / p.hop + 1) : 0;
-        CUtensorMap tmap;
-        bool have_map = false;
-        if (n_clusters > 0 && n_read > 0 && encode_tiled_fn()) {
-            const cuuint64_t e8 = iq_b / 8;
-            const cuuint64_t gdim[3] = { (cuuint64_t)k->n2 * e8, (cuuint64_t)k->n1, (cuuint64_t)n_read };
-            const cuuint64_t gstr[2] = { (cuuint64_t)k->n2 * iq_b, (cuuint64_t)p.hop * iq_b };
-            const cuuint32_t box[3] = { (cuuint32_t)(kLargeC * e8), (cuuint32_t)k->n1, 1 };
-            const cuuint32_t estr[3] = { 1, 1, 1 };
-            void* gaddr = (char*)const_cast<void*>(d_iq) + p.start_sample * iq_b;
-            have_map = gstr[1] < (1ull << 40) &&
-                       encode_tiled_fn()(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT64, 3, gaddr, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                         CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-        }
-        if (have_map) {
-            const uint64_t use = std::min<uint64_t>((uint64_t)n_clusters, p.n_frames);
-            a.ws = nullptr;
-#if SA_ONCHIP_PROF
-            rc = ensure_scratch(ws, (size_t)use * kLargeCluster * 16 * sizeof(long long));
-            if (rc) return rc;
-            a.ws = scratch[ws];
-#endif
-            a.frame0 = 0;
-            cfg.gridDim = dim3((unsigned)(use * kLargeCluster));
-            void* cargs[] = { &a, &tmap };
-            e = cudaLaunchKernelExC(&cfg, k->fn_cluster, cargs);
-            if (e != cudaSuccess) return cuda_fail(e, "launch large_onchip_kernel");
-            launches++;
-#if SA_ONCHIP_PROF
-            if (getenv("SA_ONCHIP_PROF_DUMP")) {
-                cudaStreamSynchronize(stream);
-                std::vector<long long> h((size_t)use * kLargeCluster * 16);
-                cudaMemcpy(h.data(), scratch[ws], h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-                double sum[16] = {0};
-                for (size_t c = 0; c < (size_t)use * kLargeCluster; c++) for (int i = 0; i < 16; i++) sum[i] += (double)h[c * 16 + i];
-                const double fr = (double)p.n_frames * kLargeCluster;       // CTA-frames
-                fprintf(stderr, "onchip prof (cycles per frame, mean over CTAs):");
-                for (int i = 0; i < 9; i++) fprintf(stderr, " p%d=%.0f", i, sum[i] / fr);
-                fprintf(stderr, "\n");
-            }
-#endif
-            static const char* const dkn[] = { "cf32", "ci16", "c8", "cf64" };
-            char nm[160];
-            snprintf(nm, sizeof(nm), "large_onchip_kernel<%s,%dx%d,%s,%s> (%d-CTA clusters x %d)", prec == SA_PREC_F64 ? "double" : "float",
-                     k->n1, k->n2, dkn[dk], win ? "window" : "rect", kLargeCluster, n_clusters);
-            last_kernel = nm;
-            return SA_OK;
-        }
-    }
-    // Fused persistent kernel, opt-in (SA_LARGE_FUSED=1): both steps in one launch, work items drawn from a ticket counter,
-    // workspace = an L2-persisting ring of frames (DRAM traffic ~ the algorithmic bytes).  Measured on B200: config 5 0.84-0.86 ms
-    // against 0.78 ms for the two kernels below, FP32 65536 1.08-1.30 against 0.69 ms (without the persisting window 1.25 /
-    // 1.52 ms): the per-item device-wide fence, the ticket round trip and two CTAs per SM cost more than the saved
-    // traffic buys (profiles/r02_c5_onchip_ablation.txt).
-    {
-        const char* fused_env = getenv("SA_LARGE_FUSED");
-        const bool fused_on = fused_env ? atoi(fused_env) != 0 : false;
-        const char* ring_env = getenv("SA_LARGE_RING");
-        const char* delay_env = getenv("SA_LARGE_DELAY");
-        if (k->fn_fused && fused_on) {
-            int ring = ring_env ? atoi(ring_env) : (int)std::max<uint64_t>(24, (40ull << 20) / per_frame);
-            int delay = delay_env ? atoi(delay_env) : 12;
-            if (delay < 1) delay = 1;
-            if (ring < delay + 12) ring = delay + 12;
-            if (!l2_persist_set) {
-                cudaDeviceProp prop;
-                if (cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.persistingL2CacheMaxSize > 0) {
-                    cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)prop.persistingL2CacheMaxSize);
-                    l2_window_max = (size_t)prop.accessPolicyMaxWindowSize;
-                }
-                cudaGetLastError();
-                l2_persist_set = true;
-            }
-            const size_t ring_bytes = ((size_t)ring * per_frame + 255) & ~(size_t)255;
-            const size_t ctr_bytes = (16 + 2 * (size_t)p.n_frames * sizeof(int) + 255) & ~(size_t)255;
-            rc = ensure_scratch(ws, ring_bytes + ctr_bytes);
-            if (rc) return rc;
-            char* base_ws = (char*)scratch[ws];
-            e = cudaMemsetAsync(base_ws + ring_bytes, 0, ctr_bytes, stream);
-            if (e != cudaSuccess) return cuda_fail(e, "clear four-step counters");
-            LargeFusedArgs fa;
-            memset(&fa, 0, sizeof(fa));
-            fa.a = a;
-            fa.a.ws = base_ws;
-            fa.a.frame0 = 0;
-            fa.ticket = (unsigned long long*)(base_ws + ring_bytes);
-            fa.cols_done = (int*)(base_ws + ring_bytes + 16);
-            fa.rows_done = fa.cols_done + p.n_frames;
-            fa.ring = ring; fa.delay = delay;
-            int bps_f = 0;
-            rc = kernel_grid(k->fn_fused, k->cta_cols, k->smem_fused, &bps_f);
-            if (rc) return rc;
-            const long long n_items = ((long long)p.n_frames + delay) * (k->n2 / kLargeC + k->n1 / kLargeC);
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeAccessPolicyWindow;
-            attr[0].val.accessPolicyWindow.base_ptr = base_ws;
-            attr[0].val.accessPolicyWindow.num_bytes = std::min<size_t>(ring_bytes, l2_window_max);
-            attr[0].val.accessPolicyWindow.hitRatio = 1.0f;
-            attr[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            attr[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-            cudaLaunchConfig_t cfg;
-            memset(&cfg, 0, sizeof(cfg));
-            cfg.stream = stream;
-            const char* pers_env = getenv("SA_LARGE_PERSIST");
-            const bool pers = l2_window_max > 0 && !(pers_env && atoi(pers_env) == 0);
-            cfg.attrs = attr; cfg.numAttrs = pers ? 1 : 0;
-            cfg.gridDim = dim3((unsigned)std::min<long long>(n_items, (long long)bps_f * num_sms));
-            cfg.blockDim = dim3(k->cta_cols);
-            cfg.dynamicSmemBytes = k->smem_fused;
-            void* fargs[] = { &fa };
-            e = cudaLaunchKernelExC(&cfg, k->fn_fused, fargs);
-            if (e != cudaSuccess) return cuda_fail(e, "launch large_fused_kernel");
-            launches++;
-            static const char* const dkn[] = { "cf32", "ci16", "c8", "cf64" };
-            char nm[160];
-            snprintf(nm, sizeof(nm), "large_fused_kernel<%s,%dx%d,%s,%s> (ring %d, delay %d)", prec == SA_PREC_F64 ? "double" : "float",
-                     k->n1, k->n2, dkn[dk], win ? "window" : "rect", ring, delay);
-            last_kernel = nm;
-            return SA_OK;
-        }
-    }
-    // Two workspaces, two streams: even chunks run on the caller's stream, odd chunks on a helper stream forked
-    // from it, so that one chunk's column pass fills the SMs the other chunk's row pass leaves idle in its last
-    // wave, and workspaces small enough to stay in L2 no longer mean under-filled grids (SA_LARGE_DUAL=0 disables).
-    static const char* dual_env = getenv("SA_LARGE_DUAL");
-    static const bool dual_on = dual_env ? atoi(dual_env) != 0 : kLargeDualDefault;
-    // SA_LARGE_PERSIST=1: the workspace is declared L2-persisting for the two kernels (launch attribute access policy
-    // window, hit ratio 1, everything else streaming), so that the column kernel's A[k1][n2] stays in L2 until the row
-    // kernel has read it instead of making a DRAM round trip; needs a workspace well below the persisting carve-out
-    static const char* persist_env = getenv("SA_LARGE_PERSIST");
-    static const bool persist_on = persist_env ? atoi(persist_env) != 0 : false;
-    static const uint64_t ws_mb = getenv("SA_LARGE_WS_MB") ? (uint64_t)atoi(getenv("SA_LARGE_WS_MB"))
-                                                            : (persist_on ? 32 : (dual_on ? kLargeDualWsMb : 512));
-    if (persist_on && !l2_persist_set) {
-        cudaDeviceProp prop;
-        if (cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.persistingL2CacheMaxSize > 0) {
-            cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)prop.persistingL2CacheMaxSize);
-            l2_window_max = (size_t)prop.accessPolicyMaxWindowSize;
-        }
-        cudaGetLastError();
-        l2_persist_set = true;
-    }
-    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>(p.n_frames, (ws_mb << 20) / per_frame));
-    const bool dual = dual_on && p.n_frames > chunk;
-    const int ai = (ws == 2) ? 0 : ws - 4;                 // helper index: device API 0, host-pipeline slots 1..3
+    const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>(p.n_frames, (512ull << 20) / per_frame));
     rc = ensure_scratch(ws, chunk * per_frame);
     if (rc) return rc;
-    if (dual) {
-        rc = ensure_scratch(8 + ai, chunk * per_frame);
-        if (rc) return rc;
-        if (!large_aux[ai]) {
-            e = cudaStreamCreateWithFlags(&large_aux[ai], cudaStreamNonBlocking);
-            for (int j = 0; j < 2 && e == cudaSuccess; j++) e = cudaEventCreateWithFlags(&large_ev[ai][j], cudaEventDisableTiming);
-            if (e != cudaSuccess) return cuda_fail(e, "four-step helper stream");
-        }
-        e = cudaEventRecord(large_ev[ai][0], stream);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(large_aux[ai], large_ev[ai][0], 0);
-        if (e != cudaSuccess) return cuda_fail(e, "four-step fork");
-    }
-    e = cudaFuncSetAttribute(k->fn_cols, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_cols);
+    a.ws = scratch[ws];
+    cudaError_t e = cudaFuncSetAttribute(k->fn_cols, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_cols);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(k->fn_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_rows);
     if (e != cudaSuccess) return cuda_fail(e, "large FFT smem attribute");
-    uint64_t c = 0;
-    for (uint64_t f0 = 0; f0 < p.n_frames; f0 += chunk, c++) {
+    void* args[] = { &a };
+    for (uint64_t f0 = 0; f0 < p.n_frames; f0 += chunk) {
         const unsigned nf = (unsigned)std::min<uint64_t>(chunk, p.n_frames - f0);
-        const bool odd = dual && (c & 1);
-        cudaStream_t st = odd ? large_aux[ai] : stream;
-        a.ws = scratch[odd ? 8 + ai : ws];
         a.frame0 = (long long)f0;
-        if (persist_on && l2_window_max > 0) {
-            cudaLaunchAttribute attr[1];
-            attr[0].id = cudaLaunchAttributeAccessPolicyWindow;
-            attr[0].val.accessPolicyWindow.base_ptr = a.ws;
-            attr[0].val.accessPolicyWindow.num_bytes = std::min<size_t>((size_t)nf * per_frame, l2_window_max);
-            attr[0].val.accessPolicyWindow.hitRatio = 1.0f;
-            attr[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-            attr[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-            cudaLaunchConfig_t cfg;
-            memset(&cfg, 0, sizeof(cfg));
-            cfg.stream = st; cfg.attrs = attr; cfg.numAttrs = 1;
-            cfg.gridDim = dim3(k->n2 / kLargeC, nf); cfg.blockDim = dim3(k->cta_cols); cfg.dynamicSmemBytes = k->smem_cols;
-            e = cudaLaunchKernelExC(&cfg, k->fn_cols, args);
-            if (e != cudaSuccess) return cuda_fail(e, "launch large_cols_kernel");
-            cfg.gridDim = dim3(k->n1 / kLargeC, nf); cfg.blockDim = dim3(k->cta_rows); cfg.dynamicSmemBytes = k->smem_rows;
-            e = cudaLaunchKernelExC(&cfg, k->fn_rows, args);
-            if (e != cudaSuccess) return cuda_fail(e, "launch large_rows_kernel");
-            launches += 2;
-            continue;
-        }
-        e = cudaLaunchKernel(k->fn_cols, dim3(k->n2 / kLargeC, nf), dim3(k->cta_cols), args, k->smem_cols, st);
+        e = cudaLaunchKernel(k->fn_cols, dim3(k->n2 / kLargeC, nf), dim3(k->cta_cols), args, k->smem_cols, stream);
         if (e != cudaSuccess) return cuda_fail(e, "launch large_cols_kernel");
-        e = cudaLaunchKernel(k->fn_rows, dim3(k->n1 / kLargeC, nf), dim3(k->cta_rows), args, k->smem_rows, st);
+        e = cudaLaunchKernel(k->fn_rows, dim3(k->n1 / kLargeC, nf), dim3(k->cta_rows), args, k->smem_rows, stream);
         if (e != cudaSuccess) return cuda_fail(e, "launch large_rows_kernel");
         launches += 2;
     }
-    {
-        static const char* const dkn[] = { "cf32", "ci16", "c8", "cf64" };
-        char nm[160];
-        snprintf(nm, sizeof(nm), "large_cols_kernel+large_rows_kernel<%s,%dx%d,%s,%s>", prec == SA_PREC_F64 ? "double" : "float",
-                 k->n1, k->n2, dkn[dk], win ? "window" : "rect");
-        last_kernel = nm;
-    }
-    if (dual) {
-        e = cudaEventRecord(large_ev[ai][1], large_aux[ai]);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(stream, large_ev[ai][1], 0);
-        if (e != cudaSuccess) return cuda_fail(e, "four-step join");
-    }
+    static const char* const dkn[] = { "cf32", "ci16", "c8", "cf64" };
+    char nm[160];
+    snprintf(nm, sizeof(nm), "large_cols_kernel+large_rows_kernel<%s,%dx%d,%s,%s>", prec == SA_PREC_F64 ? "double" : "float",
+             k->n1, k->n2, dkn[dk], win ? "window" : "rect");
+    last_kernel = nm;
     return SA_OK;
 }
 
@@ -722,34 +474,18 @@ int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_sp
     }
     // transforms too large for one SM's shared memory take the four-step path
     if (p.nfft > 16384 || (prec == SA_PREC_F64 && p.nfft > 8192))
-        return launch_spectrogram_large(d_iq, n_samples, p, prec, a, d_out, stream, ws);
+        return launch_spectrogram_large(p, prec, a, stream, ws);
     // TMA-staged variant (needs every frame start 16-byte aligned), else the LDG kernel
     const uint64_t iq_b = (uint64_t)sa_bytes_per_iq(p.dtype);
     const bool aligned = ((uintptr_t)d_iq % 16 == 0) && ((p.start_sample * iq_b) % 16 == 0) && ((p.hop * iq_b) % 16 == 0);
-    static const bool no_tma = getenv("SA_NO_TMA") != nullptr;      // A/B switches for the ablations in DESIGN.md
-    static const bool no_mid = getenv("SA_NO_MID") != nullptr;
-    const SpecKernelInfo* k = (aligned && !no_tma) ? find_spec_kernel(prec, (int)p.nfft, dk, win, 1) : nullptr;
+    const SpecKernelInfo* k = aligned ? find_spec_kernel(prec, (int)p.nfft, dk, win, 1) : nullptr;
     // 4096: two radix-64 passes (one exchange) for cf32 / ci16 input; cu8 / ci8 keep the 3-pass kernel (measured)
-    static const char* r64_env = getenv("SA_R64");
-    const bool use_r64 = r64_env ? (strcmp(r64_env, "all") == 0) : (dk == DK_CF32 || dk == DK_CI16);
     // (the radix-64 kernel has its own store code: pooled launches take the small-radix-first kernel)
-    if (!k && aligned && use_r64 && !pool_mode && prec == SA_PREC_F32 && p.nfft == 4096) k = find_spec_kernel(prec, 4096, dk, win, 4);
-    // 2048: two warp-private 1024-point transforms + a radix-2 combine.  Opt-in (SA_SPLIT=1): measured against the
-    // three-pass kernel on cu8 input it executes the same 43.8 instructions per point with 29 % fewer shared-memory
-    // wavefronts and runs 2.02 vs 2.00 ms per 2^30 samples (f32 dB), 4.81 vs 4.51 ms per 2^31 (RGBA): both kernels
-    // wait on the FMA pipe, not on shared memory
-    const char* split_env = getenv("SA_SPLIT");
-    const bool use_split = split_env ? atoi(split_env) != 0 : false;
-    if (!k && aligned && use_split && !pool_mode && prec == SA_PREC_F32 && p.nfft == 2048) k = find_spec_kernel(prec, 2048, dk, win, 5);
-    if (!k && aligned && !no_mid) {                                                        // small-radix-first plan
-        // the asynchronously staged variant where it measured faster on B200 (tools/mid_pf_matrix.py): 2048 (8 frames
-        // per CTA) and 16384 (one frame owns the SM) gain 6-19 %, 4096 (4 frames per CTA) 0-10 %, 8192 loses up to 19 %.
-        // SA_MID_PF=all|none overrides.
-        static const char* pf_env = getenv("SA_MID_PF");
-        const bool pf = pf_env ? (strcmp(pf_env, "all") == 0) : (p.nfft != 8192);
-        if (pf) k = find_spec_kernel(prec, (int)p.nfft, dk, win, 3);
-        if (!k) k = find_spec_kernel(prec, (int)p.nfft, dk, win, 2);
-    }
+    if (!k && aligned && (dk == DK_CF32 || dk == DK_CI16) && !pool_mode && prec == SA_PREC_F32 && p.nfft == 4096)
+        k = find_spec_kernel(prec, 4096, dk, win, 4);
+    // small-radix-first plan, with the next frame staged asynchronously where that measured faster on B200: 2048 (8
+    // frames per CTA) and 16384 (one frame owns the SM) gain 6-19 %, 4096 (4 frames per CTA) 0-10 %, 8192 loses up to 19 %
+    if (!k && aligned) k = find_spec_kernel(prec, (int)p.nfft, dk, win, p.nfft == 8192 ? 2 : 3);
     if (!k) k = find_spec_kernel(prec, (int)p.nfft, dk, win, 0);
     if (!k) return set_error(SA_ERR_UNSUPPORTED, "no kernel for nfft %u precision %s dtype %d", p.nfft,
                              prec == SA_PREC_F64 ? "f64" : "f32", p.dtype);
@@ -775,7 +511,7 @@ int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_sp
     launches++;
     {
         static const char* const fam[] = { "spectrogram_kernel", "spectrogram_tma_kernel", "spectrogram_mid_kernel",
-                                           "spectrogram_mid_kernel(prefetch)", "spectrogram_r64_kernel", "spectrogram_split_kernel" };
+                                           "spectrogram_mid_kernel(prefetch)", "spectrogram_r64_kernel" };
         static const char* const dkn[] = { "cf32", "ci16", "c8", "cf64" };
         char nm[128];
         snprintf(nm, sizeof(nm), "%s<%s,%d,%s,%s>", fam[k->tma], prec == SA_PREC_F64 ? "double" : "float", k->n, dkn[k->dk],
@@ -947,10 +683,6 @@ Engine::~Engine() {
         if (slots[i].stream) cudaStreamDestroy(slots[i].stream);
         if (slots[i].h_in) cudaFreeHost(slots[i].h_in);
         if (slots[i].h_out) cudaFreeHost(slots[i].h_out);
-    }
-    for (int i = 0; i < 4; i++) {
-        if (large_aux[i]) cudaStreamDestroy(large_aux[i]);
-        for (int j = 0; j < 2; j++) if (large_ev[i][j]) cudaEventDestroy(large_ev[i][j]);
     }
     if (h_plan) cudaFreeHost(h_plan);
     if (plan_ev) cudaEventDestroy(plan_ev);

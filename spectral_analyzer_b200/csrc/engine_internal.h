@@ -52,7 +52,7 @@ struct AnalysisProfile {
 };
 
 constexpr int kSlots = 3;
-constexpr int kScratch = 14;
+constexpr int kScratch = 10;
 
 struct Slot {
     cudaStream_t stream = nullptr;
@@ -107,14 +107,10 @@ struct Engine {
     // device workspaces: [0] annotation plan + taps, [1] Welch plan + partial spectra, [2] four-step FFT,
     // [3] canvas / canvas dB rows, [4] signal lists of the packer / series kernels,
     // [5..7] four-step FFT workspaces of the host pipeline's slots (their chunks run concurrently on three streams)
-    // [8..11] second four-step workspace of the same callers (two-stream chunk overlap, launch_spectrogram_large)
-    // [12] FP32 rows the downconverter hands to the Welch kernels (two halves, reused batch after batch: L2 resident),
-    // [13] Welch plan + partial spectra of the helper stream's batches
+    // [8] FP32 rows the downconverter hands to the Welch kernels (two halves, reused batch after batch: L2 resident),
+    // [9] Welch plan + partial spectra of the helper stream's batches
     void* scratch[kScratch] = {};
     size_t scratch_cap[kScratch] = {};
-    cudaStream_t large_aux[4] = {};                  // helper stream per four-step caller (device API, slots 0..2)
-    cudaEvent_t large_ev[4][2] = {};                 // fork / join events of that helper stream
-    bool l2_persist_set = false; size_t l2_window_max = 0;   // persisting-L2 carve-out for the four-step workspace
     AnalysisProfile profile;                         // sa_set_analysis_config
     cudaStream_t dc_aux = nullptr;                   // annotation batches alternate between the caller's stream and this one
     cudaEvent_t dc_ev[2] = {};                       // fork / join
@@ -138,8 +134,7 @@ struct Engine {
     int mid_t1_table(int n, const void** d_tab);              // pass-1 twiddle pairs of spectrogram_mid_kernel
     // ws: index of the scratch buffer the four-step path may use as its workspace (2 for device-API calls; the
     // host pipeline passes 5 + slot so that chunks in flight on different streams never share a workspace)
-    int launch_spectrogram_large(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
-                                 const SpecArgs& base, void* d_out, cudaStream_t stream, int ws);
+    int launch_spectrogram_large(const sa_spectrogram_params& p, int prec, const SpecArgs& base, cudaStream_t stream, int ws);
     // pool_mode != 0: instead of rows, |X|^2 is reduced (1 max, 2 sum) over the pool_fpc frames of each canvas column into
     // d_out = float[n_frames / pool_fpc][nfft], which the caller has zeroed (display.cu); transforms up to 16384 points.
     // A strict_zero request transforms nothing (its rows are constants): it takes the rows path, not the pooling one.

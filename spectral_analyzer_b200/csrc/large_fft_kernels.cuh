@@ -11,7 +11,6 @@
 //                       threads store consecutive bins k = k1 + N1*k2, fft-shifted.
 // Same arithmetic contract as spectrogram_kernel (SpectralService.java:33-85, MainController.java:980-999).
 #pragma once
-#include <cuda.h>          // CUtensorMap (type only; the encoder is resolved at run time, no libcuda link)
 #include "spectrogram_tma_kernel.cuh"
 
 #ifndef SA_LARGE_ROWS_MINB
@@ -92,7 +91,7 @@ large_cols_kernel(const LargeArgs a) {
                                         blockIdx.x, smem_raw);
 }
 
-// 16-byte / 8-byte loads that bypass L1 (the workspace is written by other SMs of the same launch in the cluster kernel)
+// 16-byte / 8-byte loads of the workspace that bypass L1: each element is read once, so caching it in L1 gains nothing
 __device__ __forceinline__ float2  ld_cg(const float2* p)  { return __ldcg(p); }
 __device__ __forceinline__ double2 ld_cg(const double2* p) { return __ldcg(p); }
 
@@ -153,311 +152,8 @@ large_rows_kernel(const LargeArgs a) {
                                blockIdx.x, smem_raw, ltab);
 }
 
-// ---- fused persistent variant: both steps in ONE launch, workspace = a ring of frames that stays in L2 ----
-// The two-kernel path writes the whole chunk's A[k1][n2] to DRAM and reads it back (2.2x the algorithmic traffic; the
-// column kernel runs at 85 % of the HBM bandwidth for ITS bytes).  Chunks small enough for L2 do not help as separate
-// launches (32 launches of 512 CTAs: ramp and tail of every launch, 1.12 ms instead of 0.78), with or without an
-// L2-persisting window.  Here the CTAs of one persistent grid draw work items from a ticket counter in an order that
-// interleaves the column groups of frame f with the row groups of frame f - delay; a row item waits (acquire load of a
-// per-frame counter) until the 16 column items of its frame have published their part of A, a column item until the rows
-// of the frame that used its ring slot `ring` frames ago are done.  Every wait targets items with smaller tickets, which
-// resident CTAs hold or have finished (grid = resident CTAs), so the scheme cannot deadlock; the ring (ring x N elements)
-// is declared L2-persisting for the launch.
-struct LargeFusedArgs {
-    LargeArgs a;                 // a.ws: ring of `ring` frames
-    unsigned long long* ticket;  // zeroed before the launch
-    int* cols_done;              // [n_frames], zeroed
-    int* rows_done;              // [n_frames], zeroed
-    int ring, delay;
-};
-
-__device__ __forceinline__ int ld_acquire(const int* p) { int v; asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory"); return v; }
-// thread 0 waits for *p >= want, the CTA follows; traps instead of hanging if the producer never arrives
-__device__ __forceinline__ void wait_counter(const int* p, int want) {
-    if (threadIdx.x == 0) {
-        unsigned spins = 0;
-        while (ld_acquire(p) < want) {
-            __nanosleep(64);
-            if (++spins > (1u << 24)) __trap();
-        }
-    }
-    __syncthreads();
-}
-
-template <typename T, int N1, int N2, int DK, bool WIN>
-__global__ void __launch_bounds__(kLargeC * Geo<T, N1>::TPF, 2)
-large_fused_kernel(const LargeFusedArgs fa) {
-    static_assert(Geo<T, N1>::TPF == Geo<T, N2>::TPF, "both steps use the same CTA size");
-    constexpr int N = N1 * N2, C = kLargeC, CG = N2 / C, RG = N1 / C;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    __shared__ long long s_item;
-    const double* ltab = nullptr;
-    if constexpr (sizeof(T) == 8 && SA_F64_FAST_DB) {
-        __shared__ double s_ltab[128];
-        f64_ltab_init(s_ltab);
-        ltab = s_ltab;
-    }
-    const LargeArgs& a = fa.a;
-    const long long n_items = (a.s.n_frames + fa.delay) * (CG + RG);
-    cpx<T>* ring = reinterpret_cast<cpx<T>*>(a.ws);
-    for (;;) {
-        __syncthreads();                                      // s_item and the shared-memory buffers of the last item are free
-        if (threadIdx.x == 0) s_item = (long long)atomicAdd(fa.ticket, 1ull);
-        __syncthreads();
-        const long long item = s_item;
-        if (item >= n_items) break;
-        const long long slot = item / (CG + RG);
-        const int sub = (int)(item % (CG + RG));
-        if (sub < CG) {                                       // column group `sub` of frame `slot`
-            const long long f = slot;
-            if (f >= a.s.n_frames) continue;
-            if (f >= fa.ring) wait_counter(&fa.rows_done[f - fa.ring], RG);
-            large_cols_body<T, N1, N2, DK, WIN>(a, a.frame0 + f, ring + (size_t)(f % fa.ring) * N, sub, smem_raw);
-            __threadfence();                                  // this thread's part of A is visible device-wide ...
-            __syncthreads();
-            if (threadIdx.x == 0) atomicAdd(&fa.cols_done[f], 1);      // ... before the group is published
-        } else {                                              // row group of frame slot - delay
-            const long long f = slot - fa.delay;
-            if (f < 0) continue;
-            wait_counter(&fa.cols_done[f], CG);
-            large_rows_body<T, N1, N2>(a, a.frame0 + f, ring + (size_t)(f % fa.ring) * N, sub - CG, smem_raw, ltab);
-            __threadfence();
-            __syncthreads();                                  // every thread has read its part of the ring slot
-            if (threadIdx.x == 0) atomicAdd(&fa.rows_done[f], 1);
-        }
-    }
-}
-
-// ---- on-chip variant (N = 256 x 256): one thread-block cluster of kLargeCluster CTAs per frame ----
-// The frame never leaves the chip between the column step and the row step.  CTA `rank` of the cluster owns the
-// 32 columns n2 = 32 rank .. 32 rank + 31 in the column step and the 32 rows k1 = 32 rank .. + 31 in the row step:
-//   * X[2][256][16] (shared memory, 128 KB FP64 / 64 KB FP32) receives the CTA's raw column slice of the frame by TMA:
-//     one cp.async.bulk.tensor.3d per group of 16 columns (box 16 IQ pairs x 256 rows x 1 frame of the tensor map
-//     [frame][n1][n2] the host encodes over the capture: strides hop and 256 samples), one mbarrier per group.
-//     (First version: one 1D bulk copy per row = 512 copies of 256 B per CTA and frame -- the per-copy cost of the TMA
-//     unit, ~60-110 cycles, made the kernel 3x slower than the two-kernel path: 2.35 ms for config 5.)
-//   * column step, per group of 16 columns: thread (column, t) reads the raw points n1 = t + 16 q it alone owns,
-//     runs the 256-point FFT (registers + exchange buffer E), multiplies by W_N^(n2 k1) and writes A[k1][n2] back
-//     IN PLACE (a thread reads and writes the same 16 addresses: k1 and n1 run over the same index set);
-//   * cluster barrier; every CTA pulls its 32 rows A[k1][all 256 n2] out of the eight X buffers of the cluster with
-//     ld.shared::cluster (distributed shared memory): 16-byte loads, 256 contiguous bytes per half-warp;
-//   * cluster barrier (arrive by all, wait by warp 0 only at this point): X is free again, and warp 0 issues the TMA
-//     of the cluster's NEXT frame, which lands while the two row groups are transformed, converted to dB and stored
-//     (the other warps complete the barrier at the end of the frame).
-// DRAM traffic = the algorithmic bytes: no workspace.  Needs raw element size == sizeof(cpx<T>) (cf64 on the FP64
-// path, cf32 on the FP32 path: the raw slice and A share X) and 16-byte aligned frames; everything else takes the
-// two-kernel path above.
-constexpr int kLargeCluster = 8;
-
-__device__ __forceinline__ unsigned cluster_ctarank() { unsigned r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ unsigned cluster_id_x()    { unsigned r; asm volatile("mov.u32 %0, %%clusterid.x;" : "=r"(r)); return r; }
-__device__ __forceinline__ unsigned cluster_count_x() { unsigned r; asm volatile("mov.u32 %0, %%nclusterid.x;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait()   { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
-__device__ __forceinline__ uint32_t dsmem_addr(uint32_t local, unsigned rank) {
-    uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local), "r"(rank)); return r;
-}
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* tmap, int c0, int c1, int c2, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                 ::"r"(dst), "l"(tmap), "r"(c0), "r"(c1), "r"(c2), "r"(bar) : "memory");
-}
-__device__ __forceinline__ float2 ld_dsmem(uint32_t addr, float2*) {
-    float2 v; asm volatile("ld.shared::cluster.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr) : "memory"); return v;
-}
-__device__ __forceinline__ double2 ld_dsmem(uint32_t addr, double2*) {
-    double2 v; asm volatile("ld.shared::cluster.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(addr) : "memory"); return v;
-}
-
-template <typename T> struct OnchipGeo {
-    static constexpr int N1 = 256, N2 = 256, N = N1 * N2, C = kLargeC, COLS = N2 / kLargeCluster, GROUPS = COLS / C;
-    using G = Geo<T, 256>;
-    static constexpr int THREADS = C * G::TPF;
-    static constexpr size_t X_BYTES = (size_t)N1 * COLS * sizeof(cpx<T>);
-    static constexpr size_t E_COLS = (size_t)C * ColStride<T, 256>::value * sizeof(cpx<T>);
-    static constexpr size_t E_ROWS = (size_t)C * G::SM_ELEMS * sizeof(cpx<T>);
-    static constexpr size_t E_TILE = (size_t)N2 * (C + 1) * sizeof(T);
-    static constexpr size_t E_BYTES = ((E_COLS > E_ROWS ? (E_COLS > E_TILE ? E_COLS : E_TILE) : (E_ROWS > E_TILE ? E_ROWS : E_TILE)) + 15) & ~(size_t)15;
-    static constexpr size_t SMEM = 128 + X_BYTES + E_BYTES + GROUPS * sizeof(uint64_t);      // 128: alignment slack of X
-};
-
-// SA_ONCHIP_PROF: thread 0 of every CTA accumulates the cycles of each phase and writes them to a.ws (long long[grid][16])
-#ifndef SA_ONCHIP_PROF
-#define SA_ONCHIP_PROF 0
-#endif
-#if SA_ONCHIP_PROF
-#define OC_TICK(i) do { if (tid == 0) { const long long now_ = clock64(); prof[i] += now_ - tprev; tprev = now_; } } while (0)
-#else
-#define OC_TICK(i) do { } while (0)
-#endif
-
-template <typename T, int DK, bool WIN>
-__global__ void __launch_bounds__(OnchipGeo<T>::THREADS, sizeof(T) == 4 ? 2 : 1)
-large_onchip_kernel(const LargeArgs a, const __grid_constant__ CUtensorMap tmap) {
-    using OG = OnchipGeo<T>;
-    using G = typename OG::G;
-    using LD = Loader<T, DK>;
-    using raw_t = typename LD::raw_t;
-    static_assert(sizeof(raw_t) == sizeof(cpx<T>), "the raw slice and A[k1][n2] share the X buffer");
-    constexpr int P = G::P, TPF = G::TPF, N = OG::N, N2 = OG::N2, C = OG::C, COLS = OG::COLS, GROUPS = OG::GROUPS;
-    static_assert(GROUPS == 2 && TPF == 16 && P == 16, "geometry of the 256-point plans");
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const double* ltab = nullptr;
-    if constexpr (sizeof(T) == 8 && SA_F64_FAST_DB) {
-        __shared__ double s_ltab[128];
-        f64_ltab_init(s_ltab);
-        ltab = s_ltab;
-    }
-    unsigned char* xbase = smem_raw + ((128u - (smem_u32(smem_raw) & 127u)) & 127u);     // TMA tensor destination: 128-byte aligned
-    cpx<T>* X = reinterpret_cast<cpx<T>*>(xbase);                // [group][row][16 columns]
-    unsigned char* ebuf = xbase + OG::X_BYTES;
-    uint64_t* bars = reinterpret_cast<uint64_t*>(ebuf + OG::E_BYTES);
-    const unsigned rank = cluster_ctarank();
-    const int tid = threadIdx.x, warp = tid >> 5;
-    if (tid == 0) { mbar_init(smem_u32(&bars[0]), 1); mbar_init(smem_u32(&bars[1]), 1); }
-    __syncthreads();
-    fence_proxy_async();
-    const long long stride = cluster_count_x();
-    auto readable = [&](long long f) {
-        return f < a.s.n_frames && a.s.start_sample + (a.frame0 + f) * a.s.hop + N <= a.s.n_samples;    // MainController.java:987
-    };
-    constexpr int E8 = (int)(sizeof(raw_t) / 8);      // the tensor map counts 8-byte elements
-    auto issue = [&](long long f) {           // one thread: two boxes of 16 columns x 256 rows
-        if (tid == 0) {
-#pragma unroll
-            for (int g = 0; g < GROUPS; g++) {
-                const uint32_t bar = smem_u32(&bars[g]);
-                mbar_expect_tx(bar, (uint32_t)(OG::N1 * C * sizeof(raw_t)));
-                tma_load_3d(smem_u32(X + g * (OG::N1 * C)), &tmap, (COLS * (int)rank + C * g) * E8, 0, (int)f, bar);
-            }
-        }
-    };
-
-    const cpx<T>* tw = reinterpret_cast<const cpx<T>*>(a.s.twiddle);      // pair table of the 256-point plan
-    const cpx<T>* twn = reinterpret_cast<const cpx<T>*>(a.tw_n);
-    TwSeed<T> seed; seed.om = mk2<T>((T)1, (T)0); seed.oh = seed.om;
-    long long f = cluster_id_x();
-    if (readable(f)) issue(f);
-    uint32_t parity = 0;
-#if SA_ONCHIP_PROF
-    long long prof[16] = {0}; long long tprev = clock64();
-#endif
-    for (; f < a.s.n_frames; f += stride) {
-        const long long frame = a.frame0 + f;
-        OC_TICK(0);
-        if (!readable(f)) {          // EOF rows; every later frame of this cluster is past the end too (no copy in flight)
-            const size_t row = (size_t)frame * N + (size_t)rank * (N / kLargeCluster);
-            for (int i = tid; i < N / kLargeCluster; i += OG::THREADS) {
-                if (a.s.out_kind == OUT_F32_DB) reinterpret_cast<float*>(a.s.out)[row + i] = (float)a.s.eof_fill;
-                else if (a.s.out_kind == OUT_F64_DB) reinterpret_cast<double*>(a.s.out)[row + i] = a.s.eof_fill;
-                else reinterpret_cast<uint32_t*>(a.s.out)[row + i] = colormap_rgba((float)a.s.eof_fill, a.s);
-            }
-            continue;
-        }
-        // ---- column step: 2 groups of 16 columns, in place in X
-        {
-            const int fl = tid % C, t = tid / C;
-            cpx<T>* sm = reinterpret_cast<cpx<T>*>(ebuf) + (size_t)fl * ColStride<T, 256>::value;
-#pragma unroll 1
-            for (int g = 0; g < GROUPS; g++) {
-                mbar_wait(smem_u32(&bars[g]), parity);
-                OC_TICK(1);
-                const int n2 = COLS * (int)rank + C * g + fl;
-                cpx<T>* xc = X + g * (OG::N1 * C) + fl;
-                const raw_t* xr = reinterpret_cast<const raw_t*>(xc);
-                cpx<T> v[P];
-                if (a.s.lp.swap) {
-#pragma unroll
-                    for (int q = 0; q < P; q++) v[q] = LD::template decode<true>(a.s.lp, xr[(t + TPF * q) * C]);
-                } else {
-#pragma unroll
-                    for (int q = 0; q < P; q++) v[q] = LD::template decode<false>(a.s.lp, xr[(t + TPF * q) * C]);
-                }
-                if constexpr (WIN) {
-                    const T* w = reinterpret_cast<const T*>(a.s.window);
-#pragma unroll
-                    for (int q = 0; q < P; q++) { const T wv = __ldg(&w[(t + TPF * q) * N2 + n2]); v[q].x *= wv; v[q].y *= wv; }
-                }
-                fft_frame<T, 256, false, false, true>(v, t, sm, tw, nullptr, seed);
-                const cpx<T> step = __ldg(&twn[(n2 * TPF) & (N - 1)]);
-                cpx<T> w = __ldg(&twn[(n2 * t) & (N - 1)]);
-#pragma unroll
-                for (int q = 0; q < P; q++) {
-                    if (q > 0) {
-                        if ((q & 7) == 0) w = __ldg(&twn[(n2 * (t + TPF * q)) & (N - 1)]);
-                        else w = mk2<T>(fma_t(-w.y, step.y, w.x * step.x), fma_t(w.y, step.x, w.x * step.y));
-                    }
-                    xc[(t + TPF * q) * C] = mk2<T>(fma_t(-w.y, v[q].y, w.x * v[q].x), fma_t(w.y, v[q].x, w.x * v[q].y));
-                }
-                OC_TICK(2);
-            }
-        }
-        parity ^= 1;
-        cluster_arrive();
-        cluster_wait();                      // A[k1][n2] of the whole frame sits in the eight X buffers
-        OC_TICK(3);
-        // ---- pull this CTA's 32 rows: thread (row, t) takes n2 = t + 16 q from CTA n2 / 32
-        const int t = tid % TPF, fl = tid / TPF;
-        cpx<T> vv[GROUPS][P];
-#pragma unroll
-        for (int r = 0; r < GROUPS; r++) {
-            const int k1 = COLS * (int)rank + C * r + fl;
-#pragma unroll
-            for (int q = 0; q < P; q++) {
-                const int n2 = t + TPF * q, j = n2 & (COLS - 1);         // column j of CTA n2 / 32: group j / 16
-                vv[r][q] = ld_dsmem(dsmem_addr(smem_u32(X + (j / C) * (OG::N1 * C) + k1 * C + (j % C)), (unsigned)(n2 / COLS)), (cpx<T>*)nullptr);
-            }
-        }
-#if SA_ONCHIP_PROF
-        { double sink = 0; for (int r = 0; r < GROUPS; r++) for (int q = 0; q < P; q++) sink += (double)vv[r][q].x; if (sink == 1.2345e300) prof[15]++; }
-#endif
-        OC_TICK(4);
-        cluster_arrive();
-        const bool next = readable(f + stride);
-        if (warp == 0) {                     // once every CTA has pulled, X may take the next frame
-            cluster_wait();
-            if (next) { fence_proxy_async(); issue(f + stride); }
-        }
-        OC_TICK(5);
-        // ---- row step: 2 groups of 16 rows
-        cpx<T>* smr = reinterpret_cast<cpx<T>*>(ebuf) + (size_t)fl * G::SM_ELEMS;
-        T* tile = reinterpret_cast<T*>(ebuf);
-#pragma unroll
-        for (int r = 0; r < GROUPS; r++) {
-            fft_frame<T, 256, false, false, true>(vv[r], t, smr, tw, nullptr, seed);
-            OC_TICK(6);
-            T db[P];
-            if (a.s.db_mode == DBM_MAG_1E10) bins_to_db<T, P, DBM_MAG_1E10>(vv[r], db, ltab);
-            else bins_to_db<T, P, DBM_POWER>(vv[r], db, ltab);
-            __syncthreads();
-#pragma unroll
-            for (int q = 0; q < P; q++) tile[(t + TPF * q) * (C + 1) + fl] = db[q];
-            __syncthreads();
-            const int c = tid % C, j0 = tid / C;
-            const size_t row = (size_t)frame * N;
-            const int kbase = COLS * (int)rank + C * r + c;
-#pragma unroll 4
-            for (int k2 = j0; k2 < N2; k2 += OG::THREADS / C) {
-                const T val = tile[k2 * (C + 1) + c];
-                const size_t o = row + (size_t)((kbase + OG::N1 * k2 + N / 2) & (N - 1));     // SpectralService.java:78
-                if (a.s.out_kind == OUT_F32_DB) reinterpret_cast<float*>(a.s.out)[o] = (float)val;
-                else if (a.s.out_kind == OUT_F64_DB) reinterpret_cast<double*>(a.s.out)[o] = (double)val;
-                else reinterpret_cast<uint32_t*>(a.s.out)[o] = colormap_rgba((float)val, a.s);
-            }
-            __syncthreads();                 // the tile aliases the exchange buffer of the next transform
-            OC_TICK(7);
-        }
-        if (warp != 0) cluster_wait();
-        OC_TICK(8);
-    }
-#if SA_ONCHIP_PROF
-    if (tid == 0 && a.ws) for (int i = 0; i < 16; i++) reinterpret_cast<long long*>(a.ws)[(size_t)blockIdx.x * 16 + i] = prof[i];
-#endif
-}
-
 struct LargeKernelInfo {
-    const void* fn_cols; const void* fn_rows; const void* fn_cluster; const void* fn_fused;
-    size_t smem_cluster, smem_fused;
-    int cta_cluster;
+    const void* fn_cols; const void* fn_rows;
     int prec, n, n1, n2, dk, win;
     int cta_cols, cta_rows;
     size_t smem_cols, smem_rows;
@@ -477,18 +173,6 @@ LargeKernelInfo make_large_info(int prec) {
     const size_t ex = (size_t)kLargeC * Geo<T, N2>::SM_ELEMS * sizeof(cpx<T>);
     const size_t tile = (size_t)N2 * (kLargeC + 1) * sizeof(T);
     k.smem_rows = ex > tile ? ex : tile;
-    k.fn_cluster = nullptr; k.smem_cluster = 0; k.cta_cluster = 0;
-    k.fn_fused = nullptr; k.smem_fused = 0;
-    if constexpr (Geo<T, N1>::TPF == Geo<T, N2>::TPF) {
-        k.fn_fused = (const void*)&large_fused_kernel<T, N1, N2, DK, WIN>;
-        k.smem_fused = k.smem_cols > k.smem_rows ? k.smem_cols : k.smem_rows;
-    }
-    // on-chip cluster kernel: 256 x 256 with the raw element as wide as the complex working type
-    if constexpr (N1 == 256 && N2 == 256 && sizeof(typename Loader<T, DK>::raw_t) == sizeof(cpx<T>)) {
-        k.fn_cluster = (const void*)&large_onchip_kernel<T, DK, WIN>;
-        k.smem_cluster = OnchipGeo<T>::SMEM;
-        k.cta_cluster = OnchipGeo<T>::THREADS;
-    }
     return k;
 }
 

@@ -3,7 +3,6 @@
 #include "spectrogram_tma_kernel.cuh"
 #include "spectrogram_mid_kernel.cuh"
 #include "spectrogram_r64_kernel.cuh"
-#include "spectrogram_split_kernel.cuh"
 
 #ifndef SA_INST_PREC
 #error "compile with -DSA_INST_PREC=1|2 -DSA_INST_N=<nfft>"
@@ -30,15 +29,18 @@ struct Registrar {
         register_spec_kernel(make_spec_tma_info<float, SA_INST_N, DK_C8, false>(1));
         register_spec_kernel(make_spec_tma_info<float, SA_INST_N, DK_C8, true>(1));
 #endif
-#if SA_INST_N >= 2048
-        // small-radix-first plan with 128-bit loads, taken when the frames are 16-byte aligned
+#if SA_INST_N == 8192
+        // small-radix-first plan with 128-bit loads, taken when the frames are 16-byte aligned (at 8192 points without
+        // the next-frame staging below: it measured up to 19 % slower there)
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_CF32, false, false>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_CF32, true, false>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_CI16, false, false>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_CI16, true, false>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_C8, false, false>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_C8, true, false>());
-        // ... and with the next frame staged asynchronously (cp.async) under pass 2 and the epilogue
+#elif SA_INST_N >= 2048
+        // small-radix-first plan with 128-bit loads and the next frame staged asynchronously (cp.async) under pass 2 and
+        // the epilogue, taken when the frames are 16-byte aligned
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_CF32, false, true>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_CF32, true, true>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_CI16, false, true>());
@@ -46,23 +48,12 @@ struct Registrar {
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_C8, false, true>());
         register_spec_kernel(make_spec_mid_info<SA_INST_N, DK_C8, true, true>());
 #endif
-#if SA_INST_N == 2048
-        // two warp-private 1024-point transforms + one radix-2 combine (16-byte aligned frames)
-        register_spec_kernel(make_spec_split_info<DK_CF32, false>());
-        register_spec_kernel(make_spec_split_info<DK_CF32, true>());
-        register_spec_kernel(make_spec_split_info<DK_CI16, false>());
-        register_spec_kernel(make_spec_split_info<DK_CI16, true>());
-        register_spec_kernel(make_spec_split_info<DK_C8, false>());
-        register_spec_kernel(make_spec_split_info<DK_C8, true>());
-#endif
 #if SA_INST_N == 4096
         // two-pass radix-64 plan (default for cf32 / ci16 input with 16-byte aligned frames)
         register_spec_kernel(make_spec_r64_info<DK_CF32, false>());
         register_spec_kernel(make_spec_r64_info<DK_CF32, true>());
         register_spec_kernel(make_spec_r64_info<DK_CI16, false>());
         register_spec_kernel(make_spec_r64_info<DK_CI16, true>());
-        register_spec_kernel(make_spec_r64_info<DK_C8, false>());
-        register_spec_kernel(make_spec_r64_info<DK_C8, true>());
 #endif
 #else
         // FP64 arithmetic (cf64 input, or any input when the caller asks for SA_PREC_F64);

@@ -11,7 +11,7 @@
 // Requires 16-byte aligned frames (same condition as the other staged kernels).  Measured against the 3-pass kernel
 // (2^28..2^30 samples, hop 4096): cf32 0.898 -> 0.583 ms (55 % -> 85 % of the HBM roofline), ci16 1.29 -> 1.22 ms,
 // cu8 2.22 -> 2.49 ms (the strided 2-byte reads of the staged frame cost more than the 128-bit loads of the 3-pass
-// kernel), so it is the default for cf32 and ci16 input only (SA_R64=0 / all overrides).
+// kernel), so it is built and used for cf32 and ci16 input only.
 #pragma once
 #include "spectrogram_tma_kernel.cuh"
 

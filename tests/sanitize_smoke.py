@@ -27,17 +27,6 @@ for nfft in (64, 256, 1024, 2048, 4096, 16384, 65536):
         strong = ref > ref.max(axis=1, keepdims=True) - 40
         assert np.abs(got - ref)[strong].max() < 1e-3, (nfft, dt)
         n_checked += 1
-if not only or only == "split":       # opt-in two-warp 2048-point kernel
-    os.environ["SA_SPLIT"] = "1"
-    for dt, win in (("cf32_le", "hann"), ("cu8", "rect")):
-        raw = synth.recording(2048 * 6, dt, seed=5)
-        got = eng.spectrogram(raw, dt, 2048, 13, hop=1024, window=win)
-        assert eng.last_kernel.startswith("spectrogram_split_kernel"), eng.last_kernel
-        ref = co.spectrogram(raw, dt, 0, 2048, 1024, win, 13)
-        strong = ref > ref.max(axis=1, keepdims=True) - 40
-        assert np.abs(got - ref)[strong].max() < 1e-3, dt
-        n_checked += 1
-    os.environ["SA_SPLIT"] = "0"
 if not only or only == "f64":
     raw = synth.recording(16384 * 3, "cf64_le", seed=2)
     for nfft in (1024, 16384):

@@ -161,31 +161,23 @@ def test_linearity_and_time_shift_properties(engine):
     assert np.abs(p / e - 1).max() < 1e-4
 
 
-def test_both_1024_kernels_against_oracle(engine, tmp_path):
+def test_both_1024_kernels_against_oracle(engine):
     """The 1024-point FP32 plan has two kernels: TMA-staged frames (16-byte aligned frame starts) and
-    the LDG kernel (any alignment, or SA_NO_TMA=1).  Both are checked against the oracle; the LDG
-    kernel on aligned input runs in a subprocess because the switch is read once per process."""
-    import subprocess
-    import sys
+    the LDG kernel (any alignment).  Both are checked against the oracle.  The host pipeline copies the
+    capture from the first frame on, so an odd start sample alone still gives aligned frames; an odd
+    hop does not."""
     raw = synth.recording(1024 * 40, "cf32_le", seed=31)
     ref = co.spectrogram(raw, "cf32_le", 0, 1024, 512, "hann", 70)
-    got = engine.spectrogram(raw, "cf32_le", 1024, 70, hop=512, window="hann")          # TMA kernel
+    got = engine.spectrogram(raw, "cf32_le", 1024, 70, hop=512, window="hann")
+    assert engine.last_kernel == "spectrogram_tma_kernel<float,1024,cf32,window>"
     check_db_parity(got, ref)
     ref_odd = co.spectrogram(raw, "cf32_le", 3, 1024, 512, "hann", 70)
-    got_odd = engine.spectrogram(raw, "cf32_le", 1024, 70, hop=512, window="hann", start_sample=3)   # LDG kernel
+    got_odd = engine.spectrogram(raw, "cf32_le", 1024, 70, hop=512, window="hann", start_sample=3)
     check_db_parity(got_odd, ref_odd)
-    code = ("import numpy as np, sys; sys.path.insert(0, %r); import spectral_analyzer_b200 as sa;"
-            "from spectral_analyzer_b200 import synth; e = sa.Engine(0);"
-            "raw = synth.recording(1024 * 40, 'cf32_le', seed=31);"
-            "np.save(sys.argv[1], e.spectrogram(raw, 'cf32_le', 1024, 70, hop=512, window='hann'))"
-            % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    out = str(tmp_path / "sa_no_tma.npy")
-    env = dict(os.environ, SA_NO_TMA="1")
-    subprocess.run([sys.executable, "-c", code, out], check=True, env=env)
-    got_ldg = np.load(out)
-    check_db_parity(got_ldg, ref)
-    strong = ref > ref.max(axis=1, keepdims=True) - 40
-    assert np.abs(got_ldg - got)[strong].max() < 1e-4   # two twiddle sources, same answer to FP32 rounding
+    ref_ldg = co.spectrogram(raw, "cf32_le", 3, 1024, 513, "hann", 70)
+    got_ldg = engine.spectrogram(raw, "cf32_le", 1024, 70, hop=513, window="hann", start_sample=3)
+    assert engine.last_kernel == "spectrogram_kernel<float,1024,cf32,window>"
+    check_db_parity(got_ldg, ref_ldg)
 
 
 @pytest.mark.parametrize("cmap", ["Grayscale", "Heatmap"])
@@ -385,16 +377,14 @@ def test_last_kernel_name_reports_the_selected_variant(engine):
 
 
 @pytest.mark.parametrize("dt,prec,kind", [("cf64_le", "f64", "f64"), ("cf64_be", "f64", "f64"), ("cf32_le", "f32", "f32"), ("cf32_be", "f32", "f32")])
-def test_onchip_cluster_four_step(engine, monkeypatch, dt, prec, kind):
-    """65536 points with 16-byte aligned frames: the 8-CTA cluster kernel keeps the frame in distributed shared memory
-    (large_onchip_kernel).  More frames than resident clusters (every cluster pipelines several frames through its TMA
-    ring), 50 % overlap, two trailing EOF frames; against the oracle on a sample of frames, and the whole image
-    against the two-kernel path (SA_LARGE_ONCHIP=0)."""
+def test_four_step_65536_against_oracle(engine, dt, prec, kind):
+    """65536 points take the four-step path (large_cols_kernel + large_rows_kernel).  50 % overlap, two trailing EOF
+    frames; against the oracle on a sample of frames, then a rect window (FP32 path: no window multiply instantiated)
+    and an odd hop (frames only 8-byte aligned)."""
     nfft, hop, frames = 65536, 32768, 61
     raw = synth.recording((frames - 3) * hop + nfft, dt, seed=65)
-    monkeypatch.setenv("SA_LARGE_ONCHIP", "1")                  # opt-in: measured slower than the two-kernel path
     got = engine.spectrogram(raw, dt, nfft, frames, hop=hop, window="hann", precision=prec, out_kind=kind)
-    assert engine.last_kernel.startswith("large_onchip_kernel<%s,256x256,%s,window>" % ("double" if prec == "f64" else "float", dt[:4]))
+    assert engine.last_kernel == "large_cols_kernel+large_rows_kernel<%s,256x256,%s,window>" % ("double" if prec == "f64" else "float", dt[:4])
     assert (got[-2:] == -150.0).all()
     pick = [0, 1, 17, 40, frames - 3]
     for f in pick:
@@ -403,56 +393,29 @@ def test_onchip_cluster_four_step(engine, monkeypatch, dt, prec, kind):
             check_db_parity(got[f:f + 1], ref, strong_tol=1e-9, floor_tol=1e-6)
         else:
             check_db_parity(got[f:f + 1], ref)
-    monkeypatch.setenv("SA_LARGE_ONCHIP", "0")
-    two = engine.spectrogram(raw, dt, nfft, frames, hop=hop, window="hann", precision=prec, out_kind=kind)
-    assert engine.last_kernel.startswith("large_cols_kernel+large_rows_kernel")
-    # same arithmetic in the same order (the workspace round trip is the only difference): bit-identical
-    assert np.array_equal(got, two)
-    # third variant, opt-in as well: both steps in one persistent launch, ring of frames in L2 (a short ring and delay so
-    # that slots are reused and row items really wait for their columns)
-    monkeypatch.setenv("SA_LARGE_FUSED", "1")
-    monkeypatch.setenv("SA_LARGE_RING", "14")
-    monkeypatch.setenv("SA_LARGE_DELAY", "2")
-    fused = engine.spectrogram(raw, dt, nfft, frames, hop=hop, window="hann", precision=prec, out_kind=kind)
-    assert engine.last_kernel.startswith("large_fused_kernel")
-    assert np.array_equal(got, fused)
-    monkeypatch.delenv("SA_LARGE_FUSED")
-    # rect window on the FP32 path (no window multiply instantiated) and an unaligned start (two-kernel path again)
-    monkeypatch.setenv("SA_LARGE_ONCHIP", "1")
     if prec == "f32":
         g2 = engine.spectrogram(raw, dt, nfft, 5, precision=prec, out_kind=kind)
-        assert engine.last_kernel.startswith("large_onchip_kernel<float,256x256,cf32,rect>")
+        assert engine.last_kernel == "large_cols_kernel+large_rows_kernel<float,256x256,cf32,rect>"
         check_db_parity(g2[:1], co.spectrogram(raw, dt, 0, nfft, nfft, "rect", 1))
-        g3 = engine.spectrogram(raw, dt, nfft, 3, hop=nfft + 1, precision=prec, out_kind=kind)     # odd hop: frames 8-byte aligned only
-        assert engine.last_kernel.startswith("large_cols_kernel+large_rows_kernel")
+        g3 = engine.spectrogram(raw, dt, nfft, 3, hop=nfft + 1, precision=prec, out_kind=kind)
+        assert engine.last_kernel == "large_cols_kernel+large_rows_kernel<float,256x256,cf32,rect>"
         check_db_parity(g3[1:2], co.spectrogram(raw, dt, nfft + 1, nfft, nfft, "rect", 1))
 
 
 @pytest.mark.parametrize("dt", ["cf32_le", "cf32_be", "ci16_le", "ci16_be", "cu8", "ci8"])
 @pytest.mark.parametrize("win,hop", [("hann", 1024), ("rect", 2048)])
-def test_split_2048_kernel(engine, monkeypatch, dt, win, hop):
-    """Opt-in alternative for nfft 2048 (SA_SPLIT=1): two warp-private 1024-point transforms of the even / odd samples and
-    a radix-2 combine (spectrogram_split_kernel.cuh).  More frames than one pass of the grid, two trailing EOF rows;
-    against the oracle, against the default three-pass kernel, and through the RGBA and FP64-row epilogues."""
+def test_2048_kernels_against_oracle(engine, dt, win, hop):
+    """nfft 2048: the staged small-radix-first kernel on 16-byte aligned frames, the LDG kernel otherwise.  More frames
+    than one pass of the grid, two trailing EOF rows; against the oracle, and through the FP64-row epilogue."""
     nfft, frames = 2048, 1500
     raw = synth.recording((frames - 3) * hop + nfft, dt, seed=77)
-    monkeypatch.setenv("SA_SPLIT", "1")
     got = engine.spectrogram(raw, dt, nfft, frames, hop=hop, window=win)
-    assert engine.last_kernel.startswith("spectrogram_split_kernel<float,2048,")
+    assert engine.last_kernel.startswith("spectrogram_mid_kernel(prefetch)<float,2048,")
     assert (got[-2:] == -150.0).all()
     for f in (0, 1, 777, frames - 3):
         check_db_parity(got[f:f + 1], co.spectrogram(raw, dt, f * hop, nfft, hop, win, 1))
     g64 = engine.spectrogram(raw, dt, nfft, 40, hop=hop, window=win, out_kind="f64")
     assert np.array_equal(g64, got[:40].astype(np.float64))
-    rgba = engine.spectrogram(raw, dt, nfft, 40, hop=hop, window=win, out_kind="rgba8", colormap="Heatmap", sample_rate=2.4e6)
     odd = engine.spectrogram(raw, dt, nfft, 5, hop=hop + 1, window=win)                    # frames not 16-byte aligned
-    assert not engine.last_kernel.startswith("spectrogram_split_kernel")
-    monkeypatch.setenv("SA_SPLIT", "0")
-    three = engine.spectrogram(raw, dt, nfft, frames, hop=hop, window=win)
-    assert engine.last_kernel.startswith("spectrogram_mid_kernel")
-    strong = three > three.max(axis=1, keepdims=True) - 40
-    assert np.abs(three - got)[strong].max() < 1e-4       # two factorizations, same answer to FP32 rounding
-    rgba3 = engine.spectrogram(raw, dt, nfft, 40, hop=hop, window=win, out_kind="rgba8", colormap="Heatmap", sample_rate=2.4e6)
-    d = np.abs(rgba.astype(np.int32) - rgba3.astype(np.int32))
-    assert d.max() <= 255 and (d > 1).mean() < 1e-3       # +-1 LSB apart from pixels on a Heatmap breakpoint
+    assert engine.last_kernel.startswith("spectrogram_kernel<float,2048,")
     check_db_parity(odd[:1], co.spectrogram(raw, dt, 0, nfft, hop + 1, win, 1))

@@ -51,12 +51,9 @@ def test_register_and_stack_budgets():
     for k, v in head.items():
         assert v["REG"] <= 128 and v["STACK"] == 0 and v["LOCAL"] == 0, (k, v)
     # small-radix-first kernels (2048..16384): 512-thread CTAs need <= 128 registers, no spills
-    # (the asynchronously staged 8192-point variants -- not the default for that size, SA_MID_PF=all -- keep one or two
-    # words on the stack since the pass-1 twiddle recurrence; every shipped default is spill-free)
     for k, v in spec.items():
         if "spectrogram_mid_kernel" in k:
-            staged_8192 = "mid_kernelILi8192E" in k and k.split("EEEv")[0].endswith("ELb1")
-            assert v["REG"] <= 128 and v["STACK"] <= (16 if staged_8192 else 0), (k, v)
+            assert v["REG"] <= 128 and v["STACK"] == 0, (k, v)
     # radix-64 kernel: 64 points per thread is a deliberate 255-register design with a bounded spill
     r64 = {k: v for k, v in spec.items() if "spectrogram_r64_kernel" in k}
     assert r64 and all(v["REG"] <= 255 and v["STACK"] <= 256 for v in r64.values()), r64
