@@ -263,6 +263,26 @@ SA_API int32_t sa_render_canvas_device(sa_engine* engine, const void* d_iq, uint
                                        uint32_t canvas_h, uint64_t frames_per_column, int32_t reduce,
                                        void* d_out_rgba, void* cuda_stream);
 
+/* ---- spectrum traces: average, peak-hold and minimum-hold spectra of a capture range ----
+ * The frames are those of the spectrogram `params` describes (start_sample, hop, n_frames, window, dtype, byte
+ * order, precision, db_mode, eof_fill_db, strict_reference).  Output row r reduces frames [r*F, min((r+1)*F, n_frames)),
+ * F = frames_per_row: n_rows = ceil(n_frames / F) rows of nfft bins, fft-shifted as the spectrogram rows.  Per frame t
+ * and bin k the power P_t[k] is |X_t[k]|^2 (0 for a strict-reference decode that yields zeros), or for a frame past
+ * the end of the buffer the power whose level is eof_fill_db.  MEAN = sum P / count (EOF frames counted; over readable
+ * frames this is the Welch PSD of the full band times sum w^2), MAX = max P, MIN = min P, each written as the level
+ * 20*log10(sqrt(P) + 1e-10) (SA_DB_MAG_1E10) or 10*log10(P + 1e-20) (SA_DB_POWER) in params->out_kind (F32 or F64).
+ * F = 1 gives the spectrogram rows, F = n_frames one trace of the whole range.  Only the rows cross PCIe.
+ * out_mean / out_max / out_min: NULL = statistic not wanted (at least one non-NULL); each holds
+ * ceil(n_frames / frames_per_row) * nfft elements of params->out_kind; out_bytes is the capacity of each.
+ * SA_ERR_INVALID_ARG: frames_per_row == 0, n_frames == 0, all outputs NULL, SA_OUT_RGBA8, misaligned d_iq;
+ * SA_ERR_SMALL_OUTPUT: an output is too small.  sa_last_kernel_name names the transform kernel that ran. */
+SA_API int32_t sa_spectrum_trace(sa_engine* engine, const void* iq, uint64_t iq_bytes, const sa_spectrogram_params* params,
+                                 uint64_t frames_per_row, void* out_mean, void* out_max, void* out_min, uint64_t out_bytes);
+/* Same with DEVICE pointers, asynchronous on `cuda_stream`; d_iq aligned to one IQ pair. */
+SA_API int32_t sa_spectrum_trace_device(sa_engine* engine, const void* d_iq, uint64_t iq_bytes,
+                                        const sa_spectrogram_params* params, uint64_t frames_per_row, void* d_mean,
+                                        void* d_max, void* d_min, uint64_t out_bytes, void* cuda_stream);
+
 /* ---- downconverter output epilogues (SURVEY.md 8f N3) ----
  * sa_iq_pack: IqData.getInterleavedBinary (S/data/IqData.java:160-187): interleaved little-endian
  * float32 ((float) x) or int16 ((short)(32767 * x), Java narrowing: truncate, saturate to int, keep

@@ -51,6 +51,13 @@ public:
     // the engine's JDSP profile (sa_analysis_config: taps, delay / length rule, PSD scaling / detrend / precision)
     void setAnalysisConfig(const sa_analysis_config& c) { sa_check(sa_set_analysis_config(h_, &c)); }
     void resetAnalysisConfig() { sa_check(sa_set_analysis_config(h_, nullptr)); }
+    // spectrum traces (sa_spectrum_trace): average / peak-hold / minimum-hold spectra of groups of framesPerRow frames
+    // of the spectrogram these arguments describe; each wanted statistic is float [ceil(frames / framesPerRow)][fftSize]
+    // fft-shifted dB, the others stay empty
+    struct Traces { std::vector<float> mean, max, min; };
+    Traces spectrumTrace(const MappedByteBuffer& buffer, const std::string& datatype, int fftSize, int64_t frames,
+                         int64_t hop, int window, int64_t startSample, int64_t framesPerRow, bool wantMean = true,
+                         bool wantMax = true, bool wantMin = false) const;
 private:
     sa_engine* h_ = nullptr;
 };
@@ -59,6 +66,24 @@ struct Datatype {
     int32_t dtype = 0, big_endian = 0;
     explicit Datatype(const std::string& sigmf) { sa_check(sa_parse_datatype(sigmf.c_str(), &dtype, &big_endian)); }
 };
+
+inline Engine::Traces Engine::spectrumTrace(const MappedByteBuffer& buffer, const std::string& datatype, int fftSize,
+                                            int64_t frames, int64_t hop, int window, int64_t startSample,
+                                            int64_t framesPerRow, bool wantMean, bool wantMax, bool wantMin) const {
+    const Datatype dt(datatype);
+    sa_spectrogram_params p;
+    sa_spectrogram_params_init(&p);
+    p.dtype = dt.dtype; p.big_endian = dt.big_endian; p.nfft = (uint32_t)fftSize; p.hop = (uint64_t)hop;
+    p.window = window; p.start_sample = (uint64_t)startSample; p.n_frames = (uint64_t)frames;
+    const size_t n = framesPerRow > 0 ? (size_t)((frames + framesPerRow - 1) / framesPerRow) * (size_t)fftSize : 0;
+    Traces t;
+    if (wantMean) t.mean.resize(n);
+    if (wantMax) t.max.resize(n);
+    if (wantMin) t.min.resize(n);
+    sa_check(sa_spectrum_trace(h_, buffer.data, buffer.capacity, &p, (uint64_t)framesPerRow, wantMean ? t.mean.data() : nullptr,
+                               wantMax ? t.max.data() : nullptr, wantMin ? t.min.data() : nullptr, n * sizeof(float)));
+    return t;
+}
 
 class SpectralService {
 public:

@@ -75,6 +75,9 @@ public final class NativeSpectralEngine implements AutoCloseable {
     // int32 sa_render_canvas(engine, iq, iq_bytes, params, canvas_w, canvas_h, frames_per_column, reduce, out_rgba)
     private static final MethodHandle RENDER_CANVAS = fn("sa_render_canvas",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, JAVA_INT, JAVA_INT, JAVA_LONG, JAVA_INT, ADDRESS));
+    // int32 sa_spectrum_trace(engine, iq, iq_bytes, params, frames_per_row, out_mean, out_max, out_min, out_bytes)
+    private static final MethodHandle SPECTRUM_TRACE = fn("sa_spectrum_trace",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG));
     // int32 sa_iq_pack(engine, re, im, n, format, out)
     private static final MethodHandle IQ_PACK = fn("sa_iq_pack",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, ADDRESS));
@@ -312,6 +315,43 @@ public final class NativeSpectralEngine implements AutoCloseable {
             MemorySegment seg = MemorySegment.ofBuffer(buffer);
             check((int) RENDER_CANVAS.invoke(engine, seg, seg.byteSize(), p, canvasW, canvasH, 1L, 0 /* SA_REDUCE_NEAREST */, out));
             return out.toArray(ValueLayout.JAVA_BYTE);
+        }
+    }
+
+    /**
+     * Spectrum traces of a capture range (sa_spectrum_trace): the average (Welch PSD of the full band), peak-hold and
+     * minimum-hold spectra of groups of framesPerRow frames, fft-shifted dB rows.  Returns {mean, max, min}, each
+     * float[ceil(frames / framesPerRow)][fftSize], or null where the statistic was not wanted.
+     */
+    public float[][][] spectrumTrace(MappedByteBuffer buffer, long startSample, long frames, int fftSize, long hop,
+                                     int window, String datatype, long framesPerRow, boolean mean, boolean max,
+                                     boolean min) throws Throwable {
+        try (Arena a = Arena.ofConfined()) {
+            int[] dt = parse(a, datatype);
+            MemorySegment p = a.allocate(PARAMS);
+            PARAMS_INIT.invoke(p);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("dtype")), dt[0]);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("big_endian")), dt[1]);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("window")), window);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("nfft")), fftSize);
+            p.set(JAVA_LONG, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("start_sample")), startSample);
+            p.set(JAVA_LONG, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("hop")), hop);
+            p.set(JAVA_LONG, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("n_frames")), frames);
+            long rows = framesPerRow > 0 ? (frames + framesPerRow - 1) / framesPerRow : 0;
+            long bytes = rows * fftSize * 4;
+            boolean[] want = {mean, max, min};
+            MemorySegment[] out = new MemorySegment[3];
+            for (int s = 0; s < 3; s++) out[s] = want[s] ? a.allocate(Math.max(bytes, 4)) : MemorySegment.NULL;
+            MemorySegment seg = MemorySegment.ofBuffer(buffer);
+            check((int) SPECTRUM_TRACE.invoke(engine, seg, seg.byteSize(), p, framesPerRow, out[0], out[1], out[2], bytes));
+            float[][][] res = new float[3][][];
+            for (int s = 0; s < 3; s++) {
+                if (!want[s]) continue;
+                res[s] = new float[(int) rows][];
+                for (int r = 0; r < rows; r++)
+                    res[s][r] = out[s].asSlice((long) r * fftSize * 4, (long) fftSize * 4).toArray(ValueLayout.JAVA_FLOAT);
+            }
+            return res;
         }
     }
 

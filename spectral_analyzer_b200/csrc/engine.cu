@@ -310,8 +310,11 @@ int Engine::launch_spectrogram_large(const sa_spectrogram_params& p, int prec, c
     rc = ensure_scratch(ws, chunk * per_frame);
     if (rc) return rc;
     a.ws = scratch[ws];
+    // spectrum traces: the rows kernel reduces |X|^2 into the trace cells instead of writing rows
+    const bool pooled = base.pool_mode == POOL_TRACE;
+    const void* fn_rows = pooled ? k->fn_rows_pool : k->fn_rows;
     cudaError_t e = cudaFuncSetAttribute(k->fn_cols, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_cols);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(k->fn_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_rows);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(fn_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_rows);
     if (e != cudaSuccess) return cuda_fail(e, "large FFT smem attribute");
     void* args[] = { &a };
     for (uint64_t f0 = 0; f0 < p.n_frames; f0 += chunk) {
@@ -319,14 +322,14 @@ int Engine::launch_spectrogram_large(const sa_spectrogram_params& p, int prec, c
         a.frame0 = (long long)f0;
         e = cudaLaunchKernel(k->fn_cols, dim3(k->n2 / kLargeC, nf), dim3(k->cta_cols), args, k->smem_cols, stream);
         if (e != cudaSuccess) return cuda_fail(e, "launch large_cols_kernel");
-        e = cudaLaunchKernel(k->fn_rows, dim3(k->n1 / kLargeC, nf), dim3(k->cta_rows), args, k->smem_rows, stream);
+        e = cudaLaunchKernel(fn_rows, dim3(k->n1 / kLargeC, nf), dim3(k->cta_rows), args, k->smem_rows, stream);
         if (e != cudaSuccess) return cuda_fail(e, "launch large_rows_kernel");
         launches += 2;
     }
     static const char* const dkn[] = { "cf32", "ci16", "c8", "cf64" };
     char nm[160];
-    snprintf(nm, sizeof(nm), "large_cols_kernel+large_rows_kernel<%s,%dx%d,%s,%s>", prec == SA_PREC_F64 ? "double" : "float",
-             k->n1, k->n2, dkn[dk], win ? "window" : "rect");
+    snprintf(nm, sizeof(nm), "large_cols_kernel+large_rows_kernel%s<%s,%dx%d,%s,%s>", pooled ? "(pooled)" : "",
+             prec == SA_PREC_F64 ? "double" : "float", k->n1, k->n2, dkn[dk], win ? "window" : "rect");
     last_kernel = nm;
     return SA_OK;
 }
@@ -388,6 +391,20 @@ __global__ void strict_fill_kernel(const SpecArgs a, const int nfft) {
 
 static size_t out_elem_bytes(int out_kind) { return out_kind == SA_OUT_F64_DB ? 8 : 4; }
 
+// ceil(2^64 / d) for the multiply-high divisions of the pooled epilogues (0 for d == 1)
+unsigned long long pool_magic(uint64_t d) {
+    return d > 1 ? (unsigned long long)((((unsigned __int128)1 << 64) + (unsigned __int128)(d - 1)) / (unsigned __int128)d) : 0ull;
+}
+
+// |X|^2 whose level equals eof_fill_db: (10^(dB/20) - 1e-10)^2, or 10^(dB/10) - 1e-20 in power mode
+double eof_power(const sa_spectrogram_params& p) {
+    if (p.db_mode == SA_DB_MAG_1E10) {
+        const double lin = std::max(0.0, std::pow(10.0, p.eof_fill_db / 20.0) - 1e-10);
+        return lin * lin;
+    }
+    return std::max(0.0, std::pow(10.0, p.eof_fill_db / 10.0) - 1e-20);
+}
+
 // Validates a request and resolves precision; returns SA_OK or an error.
 int check_spec_params(const sa_spectrogram_params* p, int* prec_out) {
     if (!p) return set_error(SA_ERR_INVALID_ARG, "params is NULL");
@@ -426,7 +443,8 @@ int check_spec_params(const sa_spectrogram_params* p, int* prec_out) {
 
 // Launches the fused spectrogram kernel on device-resident samples.
 int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
-                               void* d_out, cudaStream_t stream, int ws, int pool_mode, uint64_t pool_fpc) {
+                               void* d_out, cudaStream_t stream, int ws, int pool_mode, uint64_t pool_fpc,
+                               const TraceCells* trace) {
     if (p.n_frames == 0) return SA_OK;
     const int dk = dtype_kind(p.dtype);
     const int win = (prec == SA_PREC_F64) ? 1 : (p.window != SA_WIN_RECT ? 1 : 0);
@@ -448,14 +466,22 @@ int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_sp
         a.cmap = p.colormap;
     }
     if (pool_mode) {
-        if (!can_pool(p, prec)) return set_error(SA_ERR_UNSUPPORTED, "fused pooling covers the in-SM transforms only");
+        if (pool_mode == POOL_TRACE) {
+            if (!trace || !can_trace(p)) return set_error(SA_ERR_UNSUPPORTED, "a strict_reference zero request has no trace launch");
+        } else if (!can_pool(p, prec)) {
+            return set_error(SA_ERR_UNSUPPORTED, "fused pooling covers the in-SM transforms only");
+        }
         a.pool_mode = pool_mode;
         a.pool_fpc = (long long)std::max<uint64_t>(1, pool_fpc);
-        a.pool_magic = a.pool_fpc > 1 ? (unsigned long long)((((unsigned __int128)1 << 64) + (unsigned __int128)(a.pool_fpc - 1)) / (unsigned __int128)a.pool_fpc) : 0ull;
-        // |X|^2 whose level equals eof_fill_db: (10^(dB/20) - 1e-10)^2, or 10^(dB/10) - 1e-20 in power mode
-        const double lin = p.db_mode == SA_DB_MAG_1E10 ? std::max(0.0, std::pow(10.0, p.eof_fill_db / 20.0) - 1e-10)
-                                                       : 0.0;
-        a.pool_eof = (float)(p.db_mode == SA_DB_MAG_1E10 ? lin * lin : std::max(0.0, std::pow(10.0, p.eof_fill_db / 10.0) - 1e-20));
+        a.pool_magic = pool_magic(a.pool_fpc);
+        a.pool_eof = (float)eof_power(p);
+        if (trace) {
+            for (int s = 0; s < 3; s++) a.trace_acc[s] = trace->acc[s];
+            a.trace_frame0 = (long long)trace->frame0;
+            a.trace_cpr = (long long)trace->cells_per_row;
+            a.trace_cmagic = pool_magic(trace->frames_per_cell);
+            a.trace_eof = eof_power(p);
+        }
     }
     if (strict_zero(p)) {                  // no sample is ever read
         for (uint64_t f0 = 0; f0 < p.n_frames; f0 += 65535u * 1024u) {

@@ -26,6 +26,8 @@ bool host_ptr_is_pinned(const void* p);     // pinned / registered host memory (
 int check_spec_params(const sa_spectrogram_params* p, int* prec_out);   // validates, resolves precision
 void fill_load_params(LoadParams& lp, const void* base, int dtype, int big_endian);
 uint64_t spec_bytes_per_iq(const sa_spectrogram_params& p);   // Global.getBytesPerSample, strict_reference aware
+unsigned long long pool_magic(uint64_t d);                    // ceil(2^64 / d), 0 for d == 1
+double eof_power(const sa_spectrogram_params& p);             // |X|^2 whose level is eof_fill_db
 // strict_reference: datatypes SpectralService.computeMagnitudes has no branch for decode to zeros (:60-63)
 inline bool strict_zero(const sa_spectrogram_params& p) {
     return p.strict_reference && (p.dtype == SA_CF64 || p.dtype == SA_DT_OTHER);
@@ -52,7 +54,7 @@ struct AnalysisProfile {
 };
 
 constexpr int kSlots = 3;
-constexpr int kScratch = 10;
+constexpr int kScratch = 12;
 
 struct Slot {
     cudaStream_t stream = nullptr;
@@ -90,6 +92,15 @@ private:
     bool stop_ = false;
 };
 
+// Accumulator of a spectrum trace launch (SpecArgs::trace_acc): frame f of the launch lands in the cell of accumulator
+// frame f + frame0; cells_per_row cells of min(frames_per_row, kTraceCellFrames) frames per row.
+struct TraceCells {
+    void* acc[3] = {};              // sum, max, min; nullptr = not wanted
+    uint64_t frame0 = 0;
+    uint64_t cells_per_row = 1;
+    uint64_t frames_per_cell = 1;
+};
+
 struct Engine {
     int device = 0;
     int num_sms = 0;
@@ -108,7 +119,8 @@ struct Engine {
     // [3] canvas / canvas dB rows, [4] signal lists of the packer / series kernels,
     // [5..7] four-step FFT workspaces of the host pipeline's slots (their chunks run concurrently on three streams)
     // [8] FP32 rows the downconverter hands to the Welch kernels (two halves, reused batch after batch: L2 resident),
-    // [9] Welch plan + partial spectra of the helper stream's batches
+    // [9] Welch plan + partial spectra of the helper stream's batches,
+    // [10] spectrum-trace accumulator cells, [11] spectrum-trace rows of the host entry before they cross PCIe
     void* scratch[kScratch] = {};
     size_t scratch_cap[kScratch] = {};
     AnalysisProfile profile;                         // sa_set_analysis_config
@@ -138,11 +150,16 @@ struct Engine {
     // pool_mode != 0: instead of rows, |X|^2 is reduced (1 max, 2 sum) over the pool_fpc frames of each canvas column into
     // d_out = float[n_frames / pool_fpc][nfft], which the caller has zeroed (display.cu); transforms up to 16384 points.
     // A strict_zero request transforms nothing (its rows are constants): it takes the rows path, not the pooling one.
+    // pool_mode == POOL_TRACE (spectrum traces, trace.cu): |X|^2 in the launch's precision is reduced into the cells of
+    // `trace` (SpecArgs::trace_acc), pool_fpc = frames per trace row; every transform size, the four-step ones included.
     int launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
-                           void* d_out, cudaStream_t stream, int ws = 2, int pool_mode = 0, uint64_t pool_fpc = 1);
+                           void* d_out, cudaStream_t stream, int ws = 2, int pool_mode = 0, uint64_t pool_fpc = 1,
+                           const TraceCells* trace = nullptr);
     static bool can_pool(const sa_spectrogram_params& p, int prec) {
         return p.nfft <= 16384 && !(prec == SA_PREC_F64 && p.nfft > 8192) && !strict_zero(p);
     }
+    // a trace reduces in the epilogue of every transform; strict_zero requests transform nothing (constant rows)
+    static bool can_trace(const sa_spectrogram_params& p) { return !strict_zero(p); }
     int spectrogram_host(const HostSource& src, uint64_t iq_bytes, const sa_spectrogram_params& p, int prec, void* out);
 };
 

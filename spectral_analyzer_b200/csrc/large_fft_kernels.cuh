@@ -95,8 +95,10 @@ large_cols_kernel(const LargeArgs a) {
 __device__ __forceinline__ float2  ld_cg(const float2* p)  { return __ldcg(p); }
 __device__ __forceinline__ double2 ld_cg(const double2* p) { return __ldcg(p); }
 
-// row group `rg` (C rows k1) of `frame`: N2-point FFTs of A[k1][.] from ws_frame, dB, fft-shifted store
-template <typename T, int N1, int N2>
+// row group `rg` (C rows k1) of `frame`: N2-point FFTs of A[k1][.] from ws_frame, dB, fft-shifted store.
+// POOL (spectrum traces, SpecArgs::trace_acc): the tile carries |X|^2 instead of dB and the transposed bins are reduced
+// into the frame's accumulator cell -- a separate instantiation, so that the rows path runs the code it always ran.
+template <typename T, int N1, int N2, bool POOL = false>
 __device__ __forceinline__ void large_rows_body(const LargeArgs& a, const long long frame, const cpx<T>* __restrict__ ws_frame,
                                                 const int rg, unsigned char* smem_raw, const double* ltab = nullptr) {
     using G = Geo<T, N2>;
@@ -114,11 +116,16 @@ __device__ __forceinline__ void large_rows_body(const LargeArgs& a, const long l
         for (int q = 0; q < P; q++) v[q] = ld_cg(&ws[t + TPF * q]);
         TwSeed<T> seed; seed.om = mk2<T>((T)1, (T)0); seed.oh = seed.om;
         fft_frame<T, N2, false, false, true>(v, t, sm, reinterpret_cast<const cpx<T>*>(a.tw2), nullptr, seed);
-        if (a.s.db_mode == DBM_MAG_1E10) bins_to_db<T, P, DBM_MAG_1E10>(v, db, ltab);
-        else bins_to_db<T, P, DBM_POWER>(v, db, ltab);
+        if constexpr (POOL) {
+#pragma unroll
+            for (int q = 0; q < P; q++) db[q] = fma_t(v[q].x, v[q].x, v[q].y * v[q].y);
+        } else {
+            if (a.s.db_mode == DBM_MAG_1E10) bins_to_db<T, P, DBM_MAG_1E10>(v, db, ltab);
+            else bins_to_db<T, P, DBM_POWER>(v, db, ltab);
+        }
     } else {
 #pragma unroll
-        for (int q = 0; q < P; q++) db[q] = (T)a.s.eof_fill;
+        for (int q = 0; q < P; q++) db[q] = POOL ? (T)a.s.trace_eof : (T)a.s.eof_fill;
     }
     // transpose the [C rows k1][N2 bins k2] tile so that consecutive threads hold consecutive k = k1 + N1*k2
     T* tile = reinterpret_cast<T*>(smem_raw);
@@ -127,8 +134,16 @@ __device__ __forceinline__ void large_rows_body(const LargeArgs& a, const long l
     for (int q = 0; q < P; q++) tile[(t + TPF * q) * (C + 1) + fl] = db[q];
     __syncthreads();
     const int c = threadIdx.x % C, j0 = threadIdx.x / C;
-    const size_t row = (size_t)frame * N;
     const int kbase = rg * C + c;
+    if constexpr (POOL) {
+        constexpr int PT = N2 / (THREADS / C);                    // bins per thread
+        static_assert(PT * (THREADS / C) == N2, "whole tile columns per thread");
+        trace_store<T, PT, N>(a.s, trace_cell(a.s, frame),
+                              [&](int i) { return (kbase + N1 * (j0 + i * (THREADS / C)) + N / 2) & (N - 1); },
+                              [&](int i) { return tile[(j0 + i * (THREADS / C)) * (C + 1) + c]; });
+        return;
+    }
+    const size_t row = (size_t)frame * N;
     for (int k2 = j0; k2 < N2; k2 += THREADS / C) {
         const T val = tile[k2 * (C + 1) + c];
         const size_t o = row + (size_t)((kbase + N1 * k2 + N / 2) & (N - 1));     // SpectralService.java:78
@@ -138,22 +153,23 @@ __device__ __forceinline__ void large_rows_body(const LargeArgs& a, const long l
     }
 }
 
-template <typename T, int N1, int N2>
+template <typename T, int N1, int N2, bool POOL = false>
 __global__ void __launch_bounds__(kLargeC * Geo<T, N2>::TPF, SA_LARGE_ROWS_MINB)
 large_rows_kernel(const LargeArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const double* ltab = nullptr;
-    if constexpr (sizeof(T) == 8 && SA_F64_FAST_DB) {
+    if constexpr (sizeof(T) == 8 && SA_F64_FAST_DB && !POOL) {
         __shared__ double s_ltab[128];
         f64_ltab_init(s_ltab);
         ltab = s_ltab;
     }
-    large_rows_body<T, N1, N2>(a, a.frame0 + blockIdx.y, reinterpret_cast<const cpx<T>*>(a.ws) + (size_t)blockIdx.y * (N1 * N2),
+    large_rows_body<T, N1, N2, POOL>(a, a.frame0 + blockIdx.y, reinterpret_cast<const cpx<T>*>(a.ws) + (size_t)blockIdx.y * (N1 * N2),
                                blockIdx.x, smem_raw, ltab);
 }
 
 struct LargeKernelInfo {
     const void* fn_cols; const void* fn_rows;
+    const void* fn_rows_pool;    // large_rows_kernel<.., POOL>: spectrum-trace reduction instead of rows
     int prec, n, n1, n2, dk, win;
     int cta_cols, cta_rows;
     size_t smem_cols, smem_rows;
@@ -166,6 +182,7 @@ LargeKernelInfo make_large_info(int prec) {
     LargeKernelInfo k;
     k.fn_cols = (const void*)&large_cols_kernel<T, N1, N2, DK, WIN>;
     k.fn_rows = (const void*)&large_rows_kernel<T, N1, N2>;
+    k.fn_rows_pool = (const void*)&large_rows_kernel<T, N1, N2, true>;
     k.prec = prec; k.n = N1 * N2; k.n1 = N1; k.n2 = N2; k.dk = DK; k.win = WIN ? 1 : 0;
     k.cta_cols = kLargeC * Geo<T, N1>::TPF;
     k.cta_rows = kLargeC * Geo<T, N2>::TPF;

@@ -40,14 +40,32 @@ struct SpecArgs {
     int         cmap;
     // display pooling fused into the epilogue (sa_render_canvas with MAX / MEAN): instead of a dB row per frame, |X|^2 is
     // reduced over the pool_fpc frames of a canvas column into out = float[columns][N] (fft-shifted bins, zero-initialised)
-    int         pool_mode;     // 0: rows; 1: max; 2: sum
+    int         pool_mode;     // 0: rows; 1: max; 2: sum; 3: spectrum trace (POOL_TRACE)
     float       pool_eof;      // |X|^2 whose level is eof_fill (frames past the end of the buffer)
-    long long   pool_fpc;      // frames per canvas column
+    long long   pool_fpc;      // frames per canvas column (per trace row)
     unsigned long long pool_magic;   // ceil(2^64 / pool_fpc) (0 for pool_fpc == 1): column = umul64hi(frame, magic), exact
                                      // for frame * pool_fpc < 2^64 -- no 64-bit division (F2I / I2F sequences) in the kernels
+    // spectrum traces (sa_spectrum_trace, trace.cu): |X|^2 in the launch's precision T is reduced into up to three
+    // accumulators T[cells][N] (fft-shifted bins, zero-initialised): [0] sum (red.add), [1] max and [2] min (red.max on
+    // the bit pattern, resp. on its complement).  A cell holds at most trace_kc = min(F, kTraceCellFrames) frames of ONE
+    // row: cell = row * trace_cpr + (f - row * F) / trace_kc, row = f / F, f = frame + trace_frame0.
+    void*       trace_acc[3];  // nullptr: statistic not wanted
+    long long   trace_frame0;  // frame of the accumulator that this launch's frame 0 is (host-pipeline chunks)
+    long long   trace_cpr;     // cells per row
+    unsigned long long trace_cmagic; // ceil(2^64 / trace_kc) (0 for trace_kc == 1)
+    double      trace_eof;     // |X|^2 of a frame past the end of the buffer (as pool_eof, FP64)
 };
+enum { POOL_TRACE = 3 };
+constexpr int kTraceCellFrames = 256;       // frames per accumulator cell at most: an FP32 cell sums <= 256 terms
 __device__ __forceinline__ long long pool_column(const SpecArgs& a, long long frame) {
     return a.pool_magic ? (long long)__umul64hi((unsigned long long)frame, a.pool_magic) : frame;
+}
+// accumulator cell of a frame: per frame, not per bin (two multiply-highs)
+__device__ __forceinline__ long long trace_cell(const SpecArgs& a, long long frame) {
+    const long long f = frame + a.trace_frame0;
+    const long long row = pool_column(a, f);
+    const unsigned long long r = (unsigned long long)(f - row * a.pool_fpc);
+    return row * a.trace_cpr + (long long)(a.trace_cmagic ? __umul64hi(r, a.trace_cmagic) : r);
 }
 
 // One reduction per bin and frame, 32 consecutive bins per warp instruction: the L2 atomic units see one 128-byte line
@@ -56,6 +74,35 @@ __device__ __forceinline__ long long pool_column(const SpecArgs& a, long long fr
 __device__ __forceinline__ void pool_red(float* p, float v, int mode) {
     if (mode == 1) asm volatile("red.global.max.u32 [%0], %1;" ::"l"(p), "r"(__float_as_uint(v)) : "memory");
     else asm volatile("red.global.add.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
+}
+
+// Trace reductions, statistic S (0 sum, 1 max, 2 min) in the launch's precision.  MIN keeps the zero-initialised
+// accumulator: the complement of the bit pattern reverses the order of non-negative values, so red.max of ~bits is
+// the minimum, and an untouched cell (0) never wins.
+template <int S> __device__ __forceinline__ void trace_red(float* p, float v) {
+    if constexpr (S == 0) asm volatile("red.global.add.f32 [%0], %1;" ::"l"(p), "f"(v) : "memory");
+    else asm volatile("red.global.max.u32 [%0], %1;" ::"l"(p), "r"(S == 1 ? __float_as_uint(v) : ~__float_as_uint(v)) : "memory");
+}
+template <int S> __device__ __forceinline__ void trace_red(double* p, double v) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(v);
+    if constexpr (S == 0) asm volatile("red.global.add.f64 [%0], %1;" ::"l"(p), "d"(v) : "memory");
+    else asm volatile("red.global.max.u64 [%0], %1;" ::"l"(p), "l"(S == 1 ? b : ~b) : "memory");
+}
+// one reduction per wanted statistic, bin and frame: bin idx(q) of cell `cell` takes pw(q), q < P (the power is
+// recomputed per statistic rather than held in P more registers)
+template <typename T, int P, int N, typename Idx, typename Pw>
+__device__ __forceinline__ void trace_store(const SpecArgs& a, const long long cell, Idx idx, Pw pw) {
+#pragma unroll
+    for (int s = 0; s < 3; s++) {
+        if (!a.trace_acc[s]) continue;                 // uniform
+        T* o = reinterpret_cast<T*>(a.trace_acc[s]) + (size_t)cell * N;
+#pragma unroll
+        for (int q = 0; q < P; q++) {
+            if (s == 0) trace_red<0>(&o[idx(q)], (T)pw(q));
+            else if (s == 1) trace_red<1>(&o[idx(q)], (T)pw(q));
+            else trace_red<2>(&o[idx(q)], (T)pw(q));
+        }
+    }
 }
 
 #ifndef SA_F64_FAST_DB
@@ -193,6 +240,11 @@ template <typename T, int N>
 __device__ __forceinline__ void store_fill(const SpecArgs& a, const long long frame, const int t) {
     constexpr int P = Geo<T, N>::P, TPF = Geo<T, N>::TPF;
     if (SA_POOL_EPILOGUE && a.pool_mode) {
+        if (a.pool_mode == POOL_TRACE) {
+            const T pe = (T)a.trace_eof;
+            trace_store<T, P, N>(a, trace_cell(a, frame), [&](int q) { return t + TPF * q; }, [&](int) { return pe; });
+            return;
+        }
         float* o = reinterpret_cast<float*>(a.out) + (size_t)pool_column(a, frame) * N;
 #pragma unroll
         for (int q = 0; q < P; q++) pool_red(&o[t + TPF * q], a.pool_eof, a.pool_mode);
@@ -266,8 +318,13 @@ __device__ __forceinline__ void store_row(const SpecArgs& a, const long long fra
                                           const cpx<T> (&v)[Plan<T, N>::P], const double* ltab = nullptr) {
     constexpr int P = Geo<T, N>::P, TPF = Geo<T, N>::TPF;
     if (SA_POOL_EPILOGUE && a.pool_mode) {          // |X|^2 only: the logarithm is taken once per pixel by canvas_power_kernel
-        float* o = reinterpret_cast<float*>(a.out) + (size_t)pool_column(a, frame) * N;
         const int kp = (t + N / 2) & (N - 1);
+        if (a.pool_mode == POOL_TRACE) {            // ... or once per trace bin by trace_finalize_kernel
+            trace_store<T, P, N>(a, trace_cell(a, frame), [&](int q) { return (kp + TPF * q) & (N - 1); },
+                                 [&](int q) { return fma_t(v[q].x, v[q].x, v[q].y * v[q].y); });
+            return;
+        }
+        float* o = reinterpret_cast<float*>(a.out) + (size_t)pool_column(a, frame) * N;
 #pragma unroll
         for (int q = 0; q < P; q++)
             pool_red(&o[(kp + TPF * q) & (N - 1)], (float)fma_t(v[q].x, v[q].x, v[q].y * v[q].y), a.pool_mode);

@@ -233,6 +233,37 @@ class Engine:
                                                  frames_per_column, _capi.REDUCE[reduce], out.ctypes.data))
         return out
 
+    TRACE_STATS = ("mean", "max", "min")
+
+    def spectrum_trace(self, buffer, datatype, nfft, n_frames, hop=None, window="rect", start_sample=0,
+                       frames_per_row=None, stats=("mean", "max"), out_kind="f32", **kw):
+        """Average / peak-hold / minimum-hold spectra of groups of frames_per_row frames of the spectrogram these
+        arguments describe (sa_spectrum_trace); frames_per_row=None: one row over all n_frames.  Host in, host out:
+        only the rows cross PCIe.  Returns {stat: float32 / float64 [n_rows, nfft]} for the requested stats."""
+        _, ptr, nbytes = _host_view(buffer)
+        fpr = n_frames if frames_per_row is None else frames_per_row
+        p = self.make_params(datatype, nfft, hop, window, n_frames, start_sample, out=out_kind, **kw)
+        outs = self._trace_outputs(stats, n_frames, fpr, nfft, out_kind)
+        ptrs = [outs[s].ctypes.data if s in outs else None for s in self.TRACE_STATS]
+        nb = next(iter(outs.values())).nbytes
+        _capi.check(_capi.lib().sa_spectrum_trace(self._h, ptr, nbytes, C.byref(p), fpr, *ptrs, nb))
+        return outs
+
+    def _trace_outputs(self, stats, n_frames, fpr, nfft, out_kind):
+        stats = (stats,) if isinstance(stats, str) else tuple(stats)
+        bad = [s for s in stats if s not in self.TRACE_STATS]
+        if bad or not stats:
+            raise ValueError("stats must be a non-empty subset of %s, got %r" % (self.TRACE_STATS, stats))
+        n_rows = -(-n_frames // fpr) if fpr > 0 and n_frames > 0 else 0
+        dt = np.float64 if out_kind == "f64" else np.float32
+        return {s: np.empty((n_rows, nfft), dt) for s in self.TRACE_STATS if s in stats}
+
+    def spectrum_trace_device(self, d_iq_ptr, iq_bytes, params, frames_per_row, d_mean=None, d_max=None, d_min=None,
+                              out_bytes=0, stream=0):
+        """Device-resident variant (raw device pointers; None = statistic not wanted), asynchronous on `stream`."""
+        _capi.check(_capi.lib().sa_spectrum_trace_device(self._h, d_iq_ptr, iq_bytes, C.byref(params), frames_per_row,
+                                                         d_mean, d_max, d_min, out_bytes, stream))
+
     def iq_pack(self, iq, fmt):
         """IqData.getInterleavedBinary (IqData.java:160-187): bytes of interleaved LE float32 / int16."""
         if fmt.lower() not in _capi.PACK:
