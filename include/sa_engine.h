@@ -283,6 +283,31 @@ SA_API int32_t sa_spectrum_trace_device(sa_engine* engine, const void* d_iq, uin
                                         const sa_spectrogram_params* params, uint64_t frames_per_row, void* d_mean,
                                         void* d_max, void* d_min, uint64_t out_bytes, void* cuda_stream);
 
+/* ---- persistence spectrum: per-bin histograms of spectrogram levels over a capture range ----
+ * The frames are those of the spectrogram `params` describes (start_sample, hop, n_frames, window, dtype, byte order,
+ * precision, db_mode, eof_fill_db, strict_reference); params->out_kind, colormap, sample_rate, min_db and max_db are
+ * ignored, the level range is [min_db, max_db) of the arguments.  Per frame t and bin k, d[t][k] is the value the
+ * spectrogram row holds: the FP32 dB value on FP32 launches, the FP64 value on FP64 launches, eof_fill_db (rounded to
+ * the launch's precision) for frames past the end of the buffer, -200 dB for strict-reference zero decodes.  In the
+ * launch's precision, each operation rounded on its own (no FMA contraction):
+ *   u     = (d - min_db) * s,   s = n_levels / (max_db - min_db)   (min_db and s computed in FP64, then rounded)
+ *   level = u >= 1 ? (int)min(u, n_levels - 1) : 0   (below the range and NaN: level 0, above it: n_levels - 1)
+ *   counts[level][(k + nfft/2) % nfft] += 1           (bins fft-shifted as the spectrogram rows; level 0 = lowest)
+ * Every column sums to n_frames (EOF frames are counted), and the counts are exactly the histogram of the engine's own
+ * dB rows for the same request.  Only the counts cross PCIe.
+ * out_counts: n_levels * nfft uint32, level-major; out_bytes is its capacity in bytes.
+ * SA_ERR_INVALID_ARG: n_levels outside 2..256, min_db / max_db not finite or max_db <= min_db, n_frames == 0,
+ * n_frames > 0xFFFFFFFF (counts are uint32), NULL output, misaligned d_iq, or what sa_spectrogram refuses for F32
+ * rows of the same request;
+ * SA_ERR_SMALL_OUTPUT: the output is too small.  sa_last_kernel_name names the transform and histogram kernels. */
+SA_API int32_t sa_spectrum_persistence(sa_engine* engine, const void* iq, uint64_t iq_bytes,
+                                       const sa_spectrogram_params* params, uint32_t n_levels, double min_db,
+                                       double max_db, uint32_t* out_counts, uint64_t out_bytes);
+/* Same with DEVICE pointers, asynchronous on `cuda_stream`; d_iq aligned to one IQ pair. */
+SA_API int32_t sa_spectrum_persistence_device(sa_engine* engine, const void* d_iq, uint64_t iq_bytes,
+                                              const sa_spectrogram_params* params, uint32_t n_levels, double min_db,
+                                              double max_db, uint32_t* d_counts, uint64_t out_bytes, void* cuda_stream);
+
 /* ---- downconverter output epilogues (SURVEY.md 8f N3) ----
  * sa_iq_pack: IqData.getInterleavedBinary (S/data/IqData.java:160-187): interleaved little-endian
  * float32 ((float) x) or int16 ((short)(32767 * x), Java narrowing: truncate, saturate to int, keep

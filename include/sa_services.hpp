@@ -58,6 +58,12 @@ public:
     Traces spectrumTrace(const MappedByteBuffer& buffer, const std::string& datatype, int fftSize, int64_t frames,
                          int64_t hop, int window, int64_t startSample, int64_t framesPerRow, bool wantMean = true,
                          bool wantMax = true, bool wantMin = false) const;
+    // persistence spectrum (sa_spectrum_persistence): per fft-shifted bin, how many of the frames of the spectrogram
+    // these arguments describe landed on each of nLevels dB levels of [minDb, maxDb); uint32 [nLevels][fftSize],
+    // level 0 the lowest, every column summing to frames
+    std::vector<uint32_t> spectrumPersistence(const MappedByteBuffer& buffer, const std::string& datatype, int fftSize,
+                                              int64_t frames, int64_t hop, int window, int64_t startSample, int nLevels,
+                                              double minDb, double maxDb) const;
 private:
     sa_engine* h_ = nullptr;
 };
@@ -83,6 +89,21 @@ inline Engine::Traces Engine::spectrumTrace(const MappedByteBuffer& buffer, cons
     sa_check(sa_spectrum_trace(h_, buffer.data, buffer.capacity, &p, (uint64_t)framesPerRow, wantMean ? t.mean.data() : nullptr,
                                wantMax ? t.max.data() : nullptr, wantMin ? t.min.data() : nullptr, n * sizeof(float)));
     return t;
+}
+
+inline std::vector<uint32_t> Engine::spectrumPersistence(const MappedByteBuffer& buffer, const std::string& datatype,
+                                                         int fftSize, int64_t frames, int64_t hop, int window,
+                                                         int64_t startSample, int nLevels, double minDb,
+                                                         double maxDb) const {
+    const Datatype dt(datatype);
+    sa_spectrogram_params p;
+    sa_spectrogram_params_init(&p);
+    p.dtype = dt.dtype; p.big_endian = dt.big_endian; p.nfft = (uint32_t)fftSize; p.hop = (uint64_t)hop;
+    p.window = window; p.start_sample = (uint64_t)startSample; p.n_frames = (uint64_t)frames;
+    std::vector<uint32_t> counts(nLevels > 0 && fftSize > 0 ? (size_t)nLevels * (size_t)fftSize : 0);
+    sa_check(sa_spectrum_persistence(h_, buffer.data, buffer.capacity, &p, (uint32_t)nLevels, minDb, maxDb, counts.data(),
+                                     counts.size() * sizeof(uint32_t)));
+    return counts;
 }
 
 class SpectralService {

@@ -78,6 +78,10 @@ public final class NativeSpectralEngine implements AutoCloseable {
     // int32 sa_spectrum_trace(engine, iq, iq_bytes, params, frames_per_row, out_mean, out_max, out_min, out_bytes)
     private static final MethodHandle SPECTRUM_TRACE = fn("sa_spectrum_trace",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, JAVA_LONG, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG));
+    // int32 sa_spectrum_persistence(engine, iq, iq_bytes, params*, n_levels, min_db, max_db, out_counts, out_bytes)
+    private static final MethodHandle SPECTRUM_PERSISTENCE = fn("sa_spectrum_persistence",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS, JAVA_INT, JAVA_DOUBLE, JAVA_DOUBLE, ADDRESS,
+                                  JAVA_LONG));
     // int32 sa_iq_pack(engine, re, im, n, format, out)
     private static final MethodHandle IQ_PACK = fn("sa_iq_pack",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, ADDRESS));
@@ -351,6 +355,37 @@ public final class NativeSpectralEngine implements AutoCloseable {
                 for (int r = 0; r < rows; r++)
                     res[s][r] = out[s].asSlice((long) r * fftSize * 4, (long) fftSize * 4).toArray(ValueLayout.JAVA_FLOAT);
             }
+            return res;
+        }
+    }
+
+    /**
+     * Persistence spectrum of a capture range (sa_spectrum_persistence): per fft-shifted bin, how many of the frames
+     * landed on each of nLevels dB levels of [minDb, maxDb) (below the range: level 0, above it: the top level).
+     * Returns int[nLevels][fftSize], level 0 the lowest; every column sums to frames.  The counts are UNSIGNED 32-bit
+     * values held in Java ints: read them with Integer.toUnsignedLong when frames may exceed Integer.MAX_VALUE.
+     */
+    public int[][] spectrumPersistence(MappedByteBuffer buffer, long startSample, long frames, int fftSize, long hop,
+                                       int window, String datatype, int nLevels, double minDb, double maxDb)
+            throws Throwable {
+        try (Arena a = Arena.ofConfined()) {
+            int[] dt = parse(a, datatype);
+            MemorySegment p = a.allocate(PARAMS);
+            PARAMS_INIT.invoke(p);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("dtype")), dt[0]);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("big_endian")), dt[1]);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("window")), window);
+            p.set(JAVA_INT, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("nfft")), fftSize);
+            p.set(JAVA_LONG, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("start_sample")), startSample);
+            p.set(JAVA_LONG, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("hop")), hop);
+            p.set(JAVA_LONG, PARAMS.byteOffset(MemoryLayout.PathElement.groupElement("n_frames")), frames);
+            long bytes = (long) Math.max(nLevels, 0) * fftSize * 4;
+            MemorySegment out = a.allocate(Math.max(bytes, 4));
+            MemorySegment seg = MemorySegment.ofBuffer(buffer);
+            check((int) SPECTRUM_PERSISTENCE.invoke(engine, seg, seg.byteSize(), p, nLevels, minDb, maxDb, out, bytes));
+            int[][] res = new int[nLevels][];
+            for (int l = 0; l < nLevels; l++)
+                res[l] = out.asSlice((long) l * fftSize * 4, (long) fftSize * 4).toArray(ValueLayout.JAVA_INT);
             return res;
         }
     }

@@ -105,6 +105,10 @@ def lib():
     L.sa_render_canvas_device.argtypes = [vp, vp, u64, C.POINTER(SpectrogramParams), u32, u32, u64, i32, vp, vp]
     L.sa_spectrum_trace.argtypes = [vp, vp, u64, C.POINTER(SpectrogramParams), u64, vp, vp, vp, u64]
     L.sa_spectrum_trace_device.argtypes = [vp, vp, u64, C.POINTER(SpectrogramParams), u64, vp, vp, vp, u64, vp]
+    L.sa_spectrum_persistence.argtypes = [vp, vp, u64, C.POINTER(SpectrogramParams), C.c_uint32, C.c_double, C.c_double,
+                                          vp, u64]
+    L.sa_spectrum_persistence_device.argtypes = [vp, vp, u64, C.POINTER(SpectrogramParams), C.c_uint32, C.c_double,
+                                                 C.c_double, vp, u64, vp]
     L.sa_iq_pack.argtypes = [vp, dp, dp, u64, i32, vp]
     L.sa_analysis_series.argtypes = [vp, dp, dp, u64, dbl, dbl, dbl, dbl, dp, dp]
     pu64 = C.POINTER(u64)

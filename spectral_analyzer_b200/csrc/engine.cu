@@ -312,7 +312,8 @@ int Engine::launch_spectrogram_large(const sa_spectrogram_params& p, int prec, c
     a.ws = scratch[ws];
     // spectrum traces: the rows kernel reduces |X|^2 into the trace cells instead of writing rows
     const bool pooled = base.pool_mode == POOL_TRACE;
-    const void* fn_rows = pooled ? k->fn_rows_pool : k->fn_rows;
+    // persistence spectra: the rows kernel's level instantiation writes one-byte levels instead of dB
+    const void* fn_rows = pooled ? k->fn_rows_pool : base.out_kind == OUT_LEVEL8 ? k->fn_rows_level : k->fn_rows;
     cudaError_t e = cudaFuncSetAttribute(k->fn_cols, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_cols);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(fn_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k->smem_rows);
     if (e != cudaSuccess) return cuda_fail(e, "large FFT smem attribute");
@@ -444,7 +445,7 @@ int check_spec_params(const sa_spectrogram_params* p, int* prec_out) {
 // Launches the fused spectrogram kernel on device-resident samples.
 int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
                                void* d_out, cudaStream_t stream, int ws, int pool_mode, uint64_t pool_fpc,
-                               const TraceCells* trace) {
+                               const TraceCells* trace, const LevelQuant* levels) {
     if (p.n_frames == 0) return SA_OK;
     const int dk = dtype_kind(p.dtype);
     const int win = (prec == SA_PREC_F64) ? 1 : (p.window != SA_WIN_RECT ? 1 : 0);
@@ -464,6 +465,12 @@ int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_sp
         a.inv_range = (float)(1.0 / (p.max_db - p.min_db));
         a.cmap_bias = (float)(-(conv + p.min_db) / (p.max_db - p.min_db));
         a.cmap = p.colormap;
+    }
+    if (p.out_kind == OUT_LEVEL8) {
+        if (!levels || pool_mode || strict_zero(p)) return set_error(SA_ERR_UNSUPPORTED, "level rows need a quantizer and a transform");
+        a.lvl_min = levels->min_db;
+        a.lvl_scale = levels->scale;
+        a.lvl_top = (double)(levels->n_levels - 1);
     }
     if (pool_mode) {
         if (pool_mode == POOL_TRACE) {
@@ -506,8 +513,9 @@ int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_sp
     const bool aligned = ((uintptr_t)d_iq % 16 == 0) && ((p.start_sample * iq_b) % 16 == 0) && ((p.hop * iq_b) % 16 == 0);
     const SpecKernelInfo* k = aligned ? find_spec_kernel(prec, (int)p.nfft, dk, win, 1) : nullptr;
     // 4096: two radix-64 passes (one exchange) for cf32 / ci16 input; cu8 / ci8 keep the 3-pass kernel (measured)
-    // (the radix-64 kernel has its own store code: pooled launches take the small-radix-first kernel)
-    if (!k && aligned && (dk == DK_CF32 || dk == DK_CI16) && !pool_mode && prec == SA_PREC_F32 && p.nfft == 4096)
+    // (the radix-64 kernel has its own store code: pooled launches and level rows take the small-radix-first kernel)
+    if (!k && aligned && (dk == DK_CF32 || dk == DK_CI16) && !pool_mode && p.out_kind != OUT_LEVEL8 && prec == SA_PREC_F32
+        && p.nfft == 4096)
         k = find_spec_kernel(prec, 4096, dk, win, 4);
     // small-radix-first plan, with the next frame staged asynchronously where that measured faster on B200: 2048 (8
     // frames per CTA) and 16384 (one frame owns the SM) gain 6-19 %, 4096 (4 frames per CTA) 0-10 %, 8192 loses up to 19 %
@@ -525,14 +533,17 @@ int Engine::launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_sp
     }
     if (rc) return rc;
     if (win) { rc = window_table(p.window, (int)p.nfft, prec, &a.window); if (rc) return rc; }
+    // level rows (persistence spectra) run the kernel's OUT_LEVEL8 instantiation
+    const void* fn = p.out_kind == OUT_LEVEL8 ? k->fn_level : k->fn;
+    if (!fn) return set_error(SA_ERR_UNSUPPORTED, "no level-row kernel for nfft %u", p.nfft);
     int bps = 0;
-    rc = kernel_grid(k->fn, k->cta, k->smem, &bps);
+    rc = kernel_grid(fn, k->cta, k->smem, &bps);
     if (rc) return rc;
     const long long n_blocks = ((long long)p.n_frames + k->fpc - 1) / k->fpc;
     const long long max_grid = (long long)bps * num_sms;
     const unsigned grid = (unsigned)std::min<long long>(n_blocks, max_grid);
     void* args[] = { &a };
-    cudaError_t e = cudaLaunchKernel(k->fn, dim3(grid), dim3(k->cta), args, k->smem, stream);
+    cudaError_t e = cudaLaunchKernel(fn, dim3(grid), dim3(k->cta), args, k->smem, stream);
     if (e != cudaSuccess) return cuda_fail(e, "launch spectrogram_kernel");
     launches++;
     {

@@ -54,7 +54,7 @@ struct AnalysisProfile {
 };
 
 constexpr int kSlots = 3;
-constexpr int kScratch = 12;
+constexpr int kScratch = 13;
 
 struct Slot {
     cudaStream_t stream = nullptr;
@@ -101,6 +101,13 @@ struct TraceCells {
     uint64_t frames_per_cell = 1;
 };
 
+// Quantizer of an OUT_LEVEL8 launch (persistence spectra, persistence.cu; SpecArgs::lvl_*)
+struct LevelQuant {
+    double min_db = 0.0;
+    double scale = 1.0;             // n_levels / (max_db - min_db), FP64
+    int n_levels = 2;
+};
+
 struct Engine {
     int device = 0;
     int num_sms = 0;
@@ -112,6 +119,8 @@ struct Engine {
     std::map<uint64_t, void*> windows;               // (prec, window, nfft) -> device table
     std::map<uint64_t, void*> misc_tables;           // FIR taps etc.
     std::map<const void*, int> occupancy;            // kernel -> resident CTAs per SM
+    // the same for kernels whose dynamic shared memory varies with the request: (kernel, bytes) -> resident CTAs per SM
+    std::map<std::pair<const void*, size_t>, int> occupancy_smem;
     std::vector<const void*> registered;             // cudaHostRegister'ed ranges
     Slot slots[kSlots];
     CopyPool* copy_pool = nullptr;                   // created on first use
@@ -120,7 +129,8 @@ struct Engine {
     // [5..7] four-step FFT workspaces of the host pipeline's slots (their chunks run concurrently on three streams)
     // [8] FP32 rows the downconverter hands to the Welch kernels (two halves, reused batch after batch: L2 resident),
     // [9] Welch plan + partial spectra of the helper stream's batches,
-    // [10] spectrum-trace accumulator cells, [11] spectrum-trace rows of the host entry before they cross PCIe
+    // [10] spectrum-trace accumulator cells, [11] spectrum-trace rows of the host entry before they cross PCIe,
+    // [12] persistence level rows of the device entry (one chunk of frames), or the histogram of the host entry
     void* scratch[kScratch] = {};
     size_t scratch_cap[kScratch] = {};
     AnalysisProfile profile;                         // sa_set_analysis_config
@@ -152,9 +162,11 @@ struct Engine {
     // A strict_zero request transforms nothing (its rows are constants): it takes the rows path, not the pooling one.
     // pool_mode == POOL_TRACE (spectrum traces, trace.cu): |X|^2 in the launch's precision is reduced into the cells of
     // `trace` (SpecArgs::trace_acc), pool_fpc = frames per trace row; every transform size, the four-step ones included.
+    // p.out_kind == OUT_LEVEL8 (persistence spectra, persistence.cu): d_out = uint8[n_frames][nfft], the level of every
+    // bin under `levels`; every transform size, the four-step ones included.
     int launch_spectrogram(const void* d_iq, uint64_t n_samples, const sa_spectrogram_params& p, int prec,
                            void* d_out, cudaStream_t stream, int ws = 2, int pool_mode = 0, uint64_t pool_fpc = 1,
-                           const TraceCells* trace = nullptr);
+                           const TraceCells* trace = nullptr, const LevelQuant* levels = nullptr);
     static bool can_pool(const sa_spectrogram_params& p, int prec) {
         return p.nfft <= 16384 && !(prec == SA_PREC_F64 && p.nfft > 8192) && !strict_zero(p);
     }

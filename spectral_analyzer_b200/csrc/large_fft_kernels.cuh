@@ -98,7 +98,7 @@ __device__ __forceinline__ double2 ld_cg(const double2* p) { return __ldcg(p); }
 // row group `rg` (C rows k1) of `frame`: N2-point FFTs of A[k1][.] from ws_frame, dB, fft-shifted store.
 // POOL (spectrum traces, SpecArgs::trace_acc): the tile carries |X|^2 instead of dB and the transposed bins are reduced
 // into the frame's accumulator cell -- a separate instantiation, so that the rows path runs the code it always ran.
-template <typename T, int N1, int N2, bool POOL = false>
+template <typename T, int N1, int N2, bool POOL = false, bool LVL = false>
 __device__ __forceinline__ void large_rows_body(const LargeArgs& a, const long long frame, const cpx<T>* __restrict__ ws_frame,
                                                 const int rg, unsigned char* smem_raw, const double* ltab = nullptr) {
     using G = Geo<T, N2>;
@@ -147,6 +147,7 @@ __device__ __forceinline__ void large_rows_body(const LargeArgs& a, const long l
     for (int k2 = j0; k2 < N2; k2 += THREADS / C) {
         const T val = tile[k2 * (C + 1) + c];
         const size_t o = row + (size_t)((kbase + N1 * k2 + N / 2) & (N - 1));     // SpectralService.java:78
+        if constexpr (LVL) { reinterpret_cast<unsigned char*>(a.s.out)[o] = db_level(val, a.s); continue; }
         if (a.s.out_kind == OUT_F32_DB) reinterpret_cast<float*>(a.s.out)[o] = (float)val;
         else if (a.s.out_kind == OUT_F64_DB) reinterpret_cast<double*>(a.s.out)[o] = (double)val;
         else reinterpret_cast<uint32_t*>(a.s.out)[o] = colormap_rgba((float)val, a.s);
@@ -167,9 +168,25 @@ large_rows_kernel(const LargeArgs a) {
                                blockIdx.x, smem_raw, ltab);
 }
 
+// level rows (OUT_LEVEL8, persistence spectra): the rows kernel with the level store instead of the dB store
+template <typename T, int N1, int N2>
+__global__ void __launch_bounds__(kLargeC * Geo<T, N2>::TPF, SA_LARGE_ROWS_MINB)
+large_rows_level_kernel(const LargeArgs a) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const double* ltab = nullptr;
+    if constexpr (sizeof(T) == 8 && SA_F64_FAST_DB) {
+        __shared__ double s_ltab[128];
+        f64_ltab_init(s_ltab);
+        ltab = s_ltab;
+    }
+    large_rows_body<T, N1, N2, false, true>(a, a.frame0 + blockIdx.y, reinterpret_cast<const cpx<T>*>(a.ws) + (size_t)blockIdx.y * (N1 * N2),
+                                            blockIdx.x, smem_raw, ltab);
+}
+
 struct LargeKernelInfo {
     const void* fn_cols; const void* fn_rows;
     const void* fn_rows_pool;    // large_rows_kernel<.., POOL>: spectrum-trace reduction instead of rows
+    const void* fn_rows_level;   // large_rows_level_kernel: OUT_LEVEL8 rows
     int prec, n, n1, n2, dk, win;
     int cta_cols, cta_rows;
     size_t smem_cols, smem_rows;
@@ -183,6 +200,7 @@ LargeKernelInfo make_large_info(int prec) {
     k.fn_cols = (const void*)&large_cols_kernel<T, N1, N2, DK, WIN>;
     k.fn_rows = (const void*)&large_rows_kernel<T, N1, N2>;
     k.fn_rows_pool = (const void*)&large_rows_kernel<T, N1, N2, true>;
+    k.fn_rows_level = (const void*)&large_rows_level_kernel<T, N1, N2>;
     k.prec = prec; k.n = N1 * N2; k.n1 = N1; k.n2 = N2; k.dk = DK; k.win = WIN ? 1 : 0;
     k.cta_cols = kLargeC * Geo<T, N1>::TPF;
     k.cta_rows = kLargeC * Geo<T, N2>::TPF;

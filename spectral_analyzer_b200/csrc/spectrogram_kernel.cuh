@@ -18,7 +18,10 @@
 
 namespace sa {
 
-enum { OUT_F32_DB = 0, OUT_F64_DB = 1, OUT_RGBA8 = 2 };
+// OUT_LEVEL8 (internal, persistence spectra, persistence.cu): one byte per bin, the level of the dB value the F32 / F64
+// row would hold, level = quantize(dB) with SpecArgs::lvl_*.  Only the *_level_kernel instantiations (store_row /
+// store_fill with LVL = true) write it, so the kernels of every other output compile to what they were.
+enum { OUT_F32_DB = 0, OUT_F64_DB = 1, OUT_RGBA8 = 2, OUT_LEVEL8 = 3 };
 enum { DBM_MAG_1E10 = 0, DBM_POWER = 1 };
 
 struct SpecArgs {
@@ -49,11 +52,24 @@ struct SpecArgs {
     // accumulators T[cells][N] (fft-shifted bins, zero-initialised): [0] sum (red.add), [1] max and [2] min (red.max on
     // the bit pattern, resp. on its complement).  A cell holds at most trace_kc = min(F, kTraceCellFrames) frames of ONE
     // row: cell = row * trace_cpr + (f - row * F) / trace_kc, row = f / F, f = frame + trace_frame0.
-    void*       trace_acc[3];  // nullptr: statistic not wanted
-    long long   trace_frame0;  // frame of the accumulator that this launch's frame 0 is (host-pipeline chunks)
-    long long   trace_cpr;     // cells per row
-    unsigned long long trace_cmagic; // ceil(2^64 / trace_kc) (0 for trace_kc == 1)
-    double      trace_eof;     // |X|^2 of a frame past the end of the buffer (as pool_eof, FP64)
+    // OUT_LEVEL8 launches are never pooled: their quantizer shares the trace fields' space, so that the arguments of
+    // every other launch keep their layout (and the kernels their register allocation).
+    union {
+        struct {
+            void*       trace_acc[3];  // nullptr: statistic not wanted
+            long long   trace_frame0;  // frame of the accumulator that this launch's frame 0 is (host-pipeline chunks)
+            long long   trace_cpr;     // cells per row
+            unsigned long long trace_cmagic; // ceil(2^64 / trace_kc) (0 for trace_kc == 1)
+            double      trace_eof;     // |X|^2 of a frame past the end of the buffer (as pool_eof, FP64)
+        };
+        // OUT_LEVEL8: u = (dB - lvl_min) * lvl_scale in the launch's precision T (both rounded to T, each operation
+        // rounded on its own), level = u >= 1 ? (int)min(u, lvl_top) : 0 (below the range and NaN: 0, above: lvl_top)
+        struct {
+            double      lvl_min;
+            double      lvl_scale;     // n_levels / (max_db - min_db)
+            double      lvl_top;       // n_levels - 1
+        };
+    };
 };
 enum { POOL_TRACE = 3 };
 constexpr int kTraceCellFrames = 256;       // frames per accumulator cell at most: an FP32 cell sums <= 256 terms
@@ -103,6 +119,19 @@ __device__ __forceinline__ void trace_store(const SpecArgs& a, const long long c
             else trace_red<2>(&o[idx(q)], (T)pw(q));
         }
     }
+}
+
+// level of a dB value (SpecArgs::lvl_*), exactly as include/sa_engine.h defines it for sa_spectrum_persistence.
+// (int)c of c in [1, 255] is the low mantissa byte of c + 2^23 (2^52) added toward zero: no F2I, the FMA pipe only.
+__device__ __forceinline__ unsigned char db_level(float d, const SpecArgs& a) {
+    const float u = __fmul_rn(__fsub_rn(d, (float)a.lvl_min), (float)a.lvl_scale);
+    const unsigned int b = __float_as_uint(__fadd_rz(fminf(u, (float)a.lvl_top), 8388608.0f));
+    return u >= 1.0f ? (unsigned char)b : 0;
+}
+__device__ __forceinline__ unsigned char db_level(double d, const SpecArgs& a) {
+    const double u = __dmul_rn(__dsub_rn(d, a.lvl_min), a.lvl_scale);
+    const unsigned int b = (unsigned int)__double2loint(__dadd_rz(fmin(u, a.lvl_top), 4503599627370496.0));
+    return u >= 1.0 ? (unsigned char)b : 0;
 }
 
 #ifndef SA_F64_FAST_DB
@@ -236,7 +265,7 @@ template <int DK> __host__ __device__ constexpr int bytes_per_iq_kind() {
 }
 
 // EOF row: frames that would read past the end of the buffer (MainController.java:994-998)
-template <typename T, int N>
+template <typename T, int N, bool LVL = false>
 __device__ __forceinline__ void store_fill(const SpecArgs& a, const long long frame, const int t) {
     constexpr int P = Geo<T, N>::P, TPF = Geo<T, N>::TPF;
     if (SA_POOL_EPILOGUE && a.pool_mode) {
@@ -259,6 +288,11 @@ __device__ __forceinline__ void store_fill(const SpecArgs& a, const long long fr
         double* o = reinterpret_cast<double*>(a.out) + row;
 #pragma unroll
         for (int q = 0; q < P; q++) o[t + TPF * q] = a.eof_fill;
+    } else if (LVL && a.out_kind == OUT_LEVEL8) {
+        unsigned char* o = reinterpret_cast<unsigned char*>(a.out) + row;
+        const unsigned char lv = db_level((T)a.eof_fill, a);
+#pragma unroll
+        for (int q = 0; q < P; q++) o[t + TPF * q] = lv;
     } else {
         uint32_t* o = reinterpret_cast<uint32_t*>(a.out) + row;
         const uint32_t px = colormap_rgba((float)a.eof_fill, a);
@@ -313,7 +347,7 @@ __device__ __forceinline__ const T* setup_window(const SpecArgs& a, unsigned cha
 
 // Epilogue of one frame: |X| -> dB (-> colour), written as the fft-shifted row
 // out[(k + N/2) % N] (SpectralService.java:76-82), k = t + TPF*q.
-template <typename T, int N>
+template <typename T, int N, bool LVL = false>
 __device__ __forceinline__ void store_row(const SpecArgs& a, const long long frame, const int t,
                                           const cpx<T> (&v)[Plan<T, N>::P], const double* ltab = nullptr) {
     constexpr int P = Geo<T, N>::P, TPF = Geo<T, N>::TPF;
@@ -349,6 +383,10 @@ __device__ __forceinline__ void store_row(const SpecArgs& a, const long long fra
         double* o = reinterpret_cast<double*>(a.out) + row;
 #pragma unroll
         for (int q = 0; q < P; q++) o[(k0 + TPF * q) & (N - 1)] = (double)db[q];
+    } else if (LVL && a.out_kind == OUT_LEVEL8) {        // the byte comes from the db[] the F32 / F64 row would store
+        unsigned char* o = reinterpret_cast<unsigned char*>(a.out) + row;
+#pragma unroll
+        for (int q = 0; q < P; q++) o[(k0 + TPF * q) & (N - 1)] = db_level(db[q], a);
     } else {
         uint32_t* o = reinterpret_cast<uint32_t*>(a.out) + row;
         const float sc = a.inv_range, bi = a.cmap_bias;
@@ -362,78 +400,18 @@ __device__ __forceinline__ void store_row(const SpecArgs& a, const long long fra
     }
 }
 
-template <typename T, int N, int DK, bool WIN>
-__global__ void __launch_bounds__(Geo<T, N>::CTA, Geo<T, N>::MINB)
-spectrogram_kernel(const SpecArgs a) {
-    using G = Geo<T, N>;
-    constexpr int P = G::P, TPF = G::TPF, FPC = G::FPC;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const double* ltab = nullptr;
-    if constexpr (sizeof(T) == 8 && SA_F64_FAST_DB) {
-        __shared__ double s_ltab[128];
-        f64_ltab_init(s_ltab);
-        ltab = s_ltab;
-    }
-    const int fl = threadIdx.x / TPF;            // frame slot in this CTA
-    const int t  = threadIdx.x % TPF;            // thread within the frame
-    cpx<T>* sm = reinterpret_cast<cpx<T>*>(smem_raw) + (size_t)fl * G::SM_ELEMS;
-    const cpx<T>* tw = setup_twiddles<T, N>(a, smem_raw);
-    const TwSeed<T> seed = load_tw_seed<T, N>(reinterpret_cast<const cpx<T>*>(a.twiddle), t);
-
-    T win_reg[G::WIN_SMEM ? 1 : P];
-    const T* win = win_reg;
-    if constexpr (WIN) win = setup_window<T, N>(a, smem_raw + G::EXTRA_WIN_OFF, win_reg, t);
-
-    const long long n_blocks = (a.n_frames + FPC - 1) / FPC;
-    // bytes of a frame that no earlier frame covers (all of it when hop >= N)
-    const int bps = bytes_per_iq_kind<DK>();
-    const int new_bytes = (int)(a.hop < N ? a.hop : N) * bps;
-    for (long long fb = blockIdx.x; fb < n_blocks; fb += gridDim.x) {
-        const long long frame = fb * FPC + fl;
-        const long long s0 = a.start_sample + frame * a.hop;            // MainController.java:984
-        {   // pull the new samples of this slot's NEXT frame into L2 while the current one is transformed
-            const long long nf = frame + (long long)gridDim.x * FPC;
-            const long long ns_end = a.start_sample + nf * a.hop + N;
-            if (nf < a.n_frames && ns_end <= a.n_samples) {
-                const char* pf = reinterpret_cast<const char*>(a.lp.base) + ns_end * bps - new_bytes;
-                for (int off = t * 128; off < new_bytes; off += TPF * 128)
-                    asm volatile("prefetch.global.L2 [%0];" ::"l"(pf + off));
-            }
-        }
-        const bool in_grid = frame < a.n_frames;
-        const bool readable = in_grid && (s0 + N <= a.n_samples);       // :987
-        cpx<T> v[P];
-        if constexpr (TPF == 32) {
-            // one frame per warp: validity is warp-uniform, so EOF rows skip the transform
-            if (!readable) {
-                if (in_grid) store_fill<T, N>(a, frame, t);
-                continue;
-            }
-        }
-        if (readable) {
-            if (a.lp.swap) {
-#pragma unroll
-                for (int q = 0; q < P; q++) v[q] = Loader<T, DK>::template load<true>(a.lp, s0 + t + TPF * q);
-            } else {
-#pragma unroll
-                for (int q = 0; q < P; q++) v[q] = Loader<T, DK>::template load<false>(a.lp, s0 + t + TPF * q);
-            }
-        } else {
-#pragma unroll
-            for (int q = 0; q < P; q++) v[q] = mk2<T>((T)0, (T)0);
-        }
-
-        fft_frame<T, N, WIN>(v, t, sm, tw, win, seed);
-
-        if (!in_grid) continue;
-        if (!readable) { store_fill<T, N>(a, frame, t); continue; }
-        store_row<T, N>(a, frame, t, v, ltab);
-    }
-}
+#define SA_KERNEL_NAME spectrogram_kernel
+#define SA_KERNEL_LVL false
+#include "spectrogram_kernel_body.inc"
+// level rows (OUT_LEVEL8, persistence spectra)
+#define SA_KERNEL_NAME spectrogram_level_kernel
+#define SA_KERNEL_LVL true
+#include "spectrogram_kernel_body.inc"
 
 // ---- registry ----
 struct SpecKernelInfo {
     const void* fn;
+    const void* fn_level;   // the same kernel writing OUT_LEVEL8 rows (nullptr: none)
     int prec;       // 1 f32, 2 f64 (SA_PREC_*)
     int n;
     int dk;
@@ -456,6 +434,7 @@ SpecKernelInfo make_spec_info(int prec) {
     using PL = Plan<T, N>;
     SpecKernelInfo k;
     k.fn = (const void*)&spectrogram_kernel<T, N, DK, WIN>;
+    k.fn_level = (const void*)&spectrogram_level_kernel<T, N, DK, WIN>;
     k.prec = prec; k.n = N; k.dk = DK; k.win = WIN ? 1 : 0;
     k.cta = G::CTA; k.fpc = G::FPC; k.minb = G::MINB; k.smem = G::SMEM_BYTES + G::TW_BYTES + (WIN ? G::WIN_BYTES : 0);
     k.p = G::P; k.np = PL::NP; k.tma = 0;

@@ -263,93 +263,20 @@ __device__ __forceinline__ void mid_setup_tables(const void* __restrict__ t1_glo
 // PF: the raw bytes of a slot's NEXT frame are staged asynchronously into the (then idle) exchange buffer while
 // pass 2 and the epilogue of the current frame run, so no global-load latency sits on the per-frame critical
 // path (it matters most where one or two frames occupy a whole SM: nfft 8192 / 16384).
-template <int N, int DK, bool WIN, bool PF>
-__global__ void __launch_bounds__(MidGeo<N>::CTA, MidGeo<N>::MINB)
-spectrogram_mid_kernel(const SpecArgs a) {
-    using G = MidGeo<N>;
-    constexpr int P = 32, R0 = G::R0, TPF = G::TPF, FPC = G::FPC;
-    constexpr int bps = bytes_per_iq_kind<DK>();
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int fl = threadIdx.x / TPF, t = threadIdx.x % TPF;
-    float2* sm = reinterpret_cast<float2*>(smem_raw) + (size_t)fl * G::SM_ELEMS;
-    TwPair<float>* t1 = reinterpret_cast<TwPair<float>*>(smem_raw + G::EX_BYTES);
-    float* wsm = reinterpret_cast<float*>(smem_raw + G::EX_BYTES + G::T1_BYTES);
-
-    // tables: pass-1 twiddle pairs [m' < 16][r < R0]; window rows in first-stage pair order
-    mid_setup_tables<N, WIN>(a.twiddle, a.window, t1, wsm);
-    __syncthreads();
-    const float* win = wsm + t * G::WROW;
-    TwSeed<float> seed;
-    {
-        const float2* root = reinterpret_cast<const float2*>(a.aux);       // W_N^j
-        seed.om = __ldg(&root[t]);
-        seed.oh = __ldg(&root[(16 * t) & (N - 1)]);
-    }
-    const TwPair<float>* t1_row = t1 + (t % R0);
-    // pass-1 twiddles by register recurrence (mid_fft_front REC1) for the sizes listed in SA_MID_REC1_MIN_N and up
-    constexpr bool kRec1 = N >= SA_MID_REC1_MIN_N;
-    TwSeed<float> seed1;
-    {
-        const TwPair<float> m0 = ldg_tw<true>(t1_row), m1 = ldg_tw<true>(t1_row + R0);
-        seed1.om = m1.lo; seed1.oh = m0.hi; seed1.q_lo = seed1.om; seed1.q_hi = seed1.om;
-    }
-
-    const long long n_blocks = (a.n_frames + FPC - 1) / FPC;
-    const int new_bytes = (int)(a.hop < N ? a.hop : N) * bps;
-    const char* base = reinterpret_cast<const char*>(a.lp.base);
-    const uint32_t sm_addr = (uint32_t)__cvta_generic_to_shared(sm);
-    auto readable_f = [&](long long fr) { return fr < a.n_frames && a.start_sample + fr * a.hop + N <= a.n_samples; };
-    if constexpr (PF) {       // prologue: stage this slot's first frame
-        const long long f0 = (long long)blockIdx.x * FPC + fl;
-        if (readable_f(f0)) mid_stage_frame<DK, N>(base + (a.start_sample + f0 * a.hop) * bps, t, sm_addr);
-    }
-    for (long long fb = blockIdx.x; fb < n_blocks; fb += gridDim.x) {
-        const long long frame = fb * FPC + fl;
-        const long long s0 = a.start_sample + frame * a.hop;              // MainController.java:984
-        const long long nf = frame + (long long)gridDim.x * FPC;          // this slot's next frame
-        if constexpr (!PF) {   // pull the new samples of the NEXT frame into L2 while the current one is transformed
-            const long long ns_end = a.start_sample + nf * a.hop + N;
-            if (nf < a.n_frames && ns_end <= a.n_samples) {
-                const char* pf = base + ns_end * bps - new_bytes;
-                for (int off = t * 128; off < new_bytes; off += TPF * 128)
-                    asm volatile("prefetch.global.L2 [%0];" ::"l"(pf + off));
-            }
-        }
-        if (frame >= a.n_frames) continue;                                // uniform over the frame's threads
-        if (s0 + N > a.n_samples) {                                       // :987, :994-998
-            store_fill<float, N>(a, frame, t);
-            if constexpr (PF) {   // nothing of this slot is in flight and every reader of the buffer is past its reads
-                if (readable_f(nf)) mid_stage_frame<DK, N>(base + (a.start_sample + nf * a.hop) * bps, t, sm_addr);
-            }
-            continue;
-        }
-
-        float2 v[P];
-        if constexpr (PF) {
-            asm volatile("cp.async.wait_group 0;" ::: "memory");           // this thread's own chunks have landed
-            const unsigned char* stage = reinterpret_cast<const unsigned char*>(sm);
-            if (a.lp.swap) mid_decode_staged<DK, N, true>(a.lp, stage, t, v);
-            else           mid_decode_staged<DK, N, false>(a.lp, stage, t, v);
-        } else {
-            if (a.lp.swap) mid_load_frame<DK, N, true>(a.lp, base + s0 * bps, t, v);
-            else           mid_load_frame<DK, N, false>(a.lp, base + s0 * bps, t, v);
-        }
-
-        mid_fft_front<N, WIN, kRec1>(v, t, fl, sm, win, t1_row, seed, &seed1);
-        if constexpr (PF) {
-            mid_sync<TPF, FPC>(fl);                                        // the exchange buffer has been read back by everyone
-            if (readable_f(nf)) mid_stage_frame<DK, N>(base + (a.start_sample + nf * a.hop) * bps, t, sm_addr);
-        }
-        mid_fft_back(v, seed);
-        store_row<float, N>(a, frame, t, v);
-    }
-}
+#define SA_KERNEL_NAME spectrogram_mid_kernel
+#define SA_KERNEL_LVL false
+#include "spectrogram_mid_kernel_body.inc"
+// level rows (OUT_LEVEL8, persistence spectra)
+#define SA_KERNEL_NAME spectrogram_mid_level_kernel
+#define SA_KERNEL_LVL true
+#include "spectrogram_mid_kernel_body.inc"
 
 template <int N, int DK, bool WIN, bool PF>
 SpecKernelInfo make_spec_mid_info() {
     using G = MidGeo<N>;
     SpecKernelInfo k;
     k.fn = (const void*)&spectrogram_mid_kernel<N, DK, WIN, PF>;
+    k.fn_level = (const void*)&spectrogram_mid_level_kernel<N, DK, WIN, PF>;
     k.prec = 1; k.n = N; k.dk = DK; k.win = WIN ? 1 : 0;
     k.cta = G::CTA; k.fpc = G::FPC; k.minb = G::MINB;
     k.smem = G::EX_BYTES + G::T1_BYTES + (WIN ? G::WIN_BYTES : 0);

@@ -164,6 +164,7 @@ SpecKernelInfo make_spec_r64_info() {
     using G = R64Geo;
     SpecKernelInfo k;
     k.fn = (const void*)&spectrogram_r64_kernel<DK, WIN>;
+    k.fn_level = nullptr;                     // its store code is its own: level rows take the mid kernel
     k.prec = 1; k.n = G::N; k.dk = DK; k.win = WIN ? 1 : 0;
     k.cta = G::CTA; k.fpc = G::FPC; k.minb = 1;
     k.smem = G::EX_BYTES + (WIN ? G::WIN_BYTES : 0) + G::BAR_BYTES;

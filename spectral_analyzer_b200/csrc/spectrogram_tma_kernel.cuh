@@ -53,90 +53,19 @@ __device__ __forceinline__ void tma_load_1d(uint32_t dst, const void* src, uint3
 }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-template <typename T, int N, int DK, bool WIN>
-__global__ void __launch_bounds__(Geo<T, N>::CTA, Geo<T, N>::MINB)
-spectrogram_tma_kernel(const SpecArgs a) {
-    using G = Geo<T, N>;
-    using LD = Loader<T, DK>;
-    using raw_t = typename LD::raw_t;
-    constexpr int P = G::P, TPF = G::TPF, FPC = G::FPC;
-    static_assert(TPF == 32 && Plan<T, N>::NP == 2, "one warp per frame, two passes");
-    constexpr uint32_t FRAME_BYTES = N * sizeof(raw_t);
-    static_assert(FRAME_BYTES <= G::SM_ELEMS * sizeof(cpx<T>), "raw frame must fit the exchange buffer");
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int fl = threadIdx.x / TPF, t = threadIdx.x % TPF;
-    cpx<T>* sm = reinterpret_cast<cpx<T>*>(smem_raw) + (size_t)fl * G::SM_ELEMS;
-    const raw_t* raw = reinterpret_cast<const raw_t*>(sm);
-    static_assert(G::TW_REC, "the TMA-staged kernel generates its pass-1 twiddles by recurrence");
-    const cpx<T>* tw = reinterpret_cast<const cpx<T>*>(a.twiddle);
-    const TwSeed<T> seed = load_tw_seed<T, N>(reinterpret_cast<const cpx<T>*>(a.twiddle), t);
-    // one mbarrier per warp, after the exchange buffers, the twiddles and the window rows
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + G::SMEM_BYTES + (WIN ? G::WIN_BYTES : 0));
-    const uint32_t bar = smem_u32(&bars[fl]);
-    const uint32_t dst = smem_u32(sm);
-
-    T win_reg[G::WIN_SMEM ? 1 : P];
-    const T* win = win_reg;
-    if constexpr (WIN) win = setup_window<T, N>(a, smem_raw + G::SMEM_BYTES, win_reg, t);
-
-    if (t == 0) mbar_init(bar, 1);
-    __syncwarp();
-    fence_proxy_async();      // barrier init visible to the async proxy
-
-    const long long n_blocks = (a.n_frames + FPC - 1) / FPC;
-    const char* base = reinterpret_cast<const char*>(a.lp.base);
-    auto frame_of = [&](long long fb) { return fb * FPC + fl; };
-    auto readable_f = [&](long long frame) {
-        return frame < a.n_frames && (a.start_sample + frame * a.hop + N <= a.n_samples);   // MainController.java:987
-    };
-    auto issue = [&](long long frame) {       // lane 0 only
-        mbar_expect_tx(bar, FRAME_BYTES);
-        tma_load_1d(dst, base + (a.start_sample + frame * a.hop) * (long long)sizeof(raw_t), FRAME_BYTES, bar);
-    };
-
-    // a CTA takes SA_TMA_BLOCKS_PER_STEP adjacent frame blocks before it strides by the grid
-    constexpr long long K = SA_TMA_BLOCKS_PER_STEP;
-    auto adv = [&](long long b) { return ((b + 1) % K != 0) ? b + 1 : b + 1 + ((long long)gridDim.x - 1) * K; };
-    long long fb = (long long)blockIdx.x * K;
-    if (fb < n_blocks && readable_f(frame_of(fb)) && t == 0) issue(frame_of(fb));
-    uint32_t parity = 0;
-    for (; fb < n_blocks; fb = adv(fb)) {
-        const long long frame = frame_of(fb);
-        const long long nfb = adv(fb);
-        const long long next = frame_of(nfb);
-        const bool next_readable = (nfb < n_blocks) && readable_f(next);
-        if (frame >= a.n_frames) continue;            // warp-uniform; a later block cannot be in range either
-        if (!readable_f(frame)) {                     // EOF row, no copy was issued for it
-            store_fill<T, N>(a, frame, t);
-            if (next_readable && t == 0) issue(next);
-            continue;
-        }
-        mbar_wait(bar, parity);
-        parity ^= 1;
-        cpx<T> v[P];
-        if (a.lp.swap) {
-#pragma unroll
-            for (int q = 0; q < P; q++) v[q] = LD::template decode<true>(a.lp, raw[t + TPF * q]);
-        } else {
-#pragma unroll
-            for (int q = 0; q < P; q++) v[q] = LD::template decode<false>(a.lp, raw[t + TPF * q]);
-        }
-        // pass 0 ends with: sync, exchange write (overwrites the raw frame), sync, exchange read
-        fft_pass<T, N, 0, WIN, true>(v, t, sm, tw, win, seed);
-        __syncwarp();                                 // every lane has read its exchange values back
-        if (next_readable && t == 0) {
-            fence_proxy_async();                      // generic-proxy accesses ordered before the async write
-            issue(next);
-        }
-        fft_pass<T, N, 1, WIN, true>(v, t, sm, tw, win, seed);
-        store_row<T, N>(a, frame, t, v);
-    }
-}
+#define SA_KERNEL_NAME spectrogram_tma_kernel
+#define SA_KERNEL_LVL false
+#include "spectrogram_tma_kernel_body.inc"
+// level rows (OUT_LEVEL8, persistence spectra)
+#define SA_KERNEL_NAME spectrogram_tma_level_kernel
+#define SA_KERNEL_LVL true
+#include "spectrogram_tma_kernel_body.inc"
 
 template <typename T, int N, int DK, bool WIN>
 SpecKernelInfo make_spec_tma_info(int prec) {
     SpecKernelInfo k = make_spec_info<T, N, DK, WIN>(prec);
     k.fn = (const void*)&spectrogram_tma_kernel<T, N, DK, WIN>;
+    k.fn_level = (const void*)&spectrogram_tma_level_kernel<T, N, DK, WIN>;
     k.smem = Geo<T, N>::SMEM_BYTES + (WIN ? Geo<T, N>::WIN_BYTES : 0) + Geo<T, N>::FPC * sizeof(uint64_t);
     k.tma = 1;
     return k;

@@ -264,6 +264,26 @@ class Engine:
         _capi.check(_capi.lib().sa_spectrum_trace_device(self._h, d_iq_ptr, iq_bytes, C.byref(params), frames_per_row,
                                                          d_mean, d_max, d_min, out_bytes, stream))
 
+    def spectrum_persistence(self, buffer, datatype, nfft, n_frames, n_levels, min_db, max_db, hop=None, window="rect",
+                             start_sample=0, **kw):
+        """Persistence spectrum (sa_spectrum_persistence): per fft-shifted bin, how many of the n_frames frames of the
+        spectrogram these arguments describe landed on each of n_levels dB levels of [min_db, max_db) (below: level 0,
+        above: the top level).  Host in, host out: only the counts cross PCIe.  Returns uint32 [n_levels, nfft], row 0
+        the lowest level; every column sums to n_frames."""
+        _, ptr, nbytes = _host_view(buffer)
+        p = self.make_params(datatype, nfft, hop, window, n_frames, start_sample, **kw)
+        out = np.empty((n_levels, nfft), np.uint32)
+        _capi.check(_capi.lib().sa_spectrum_persistence(self._h, ptr, nbytes, C.byref(p), n_levels, min_db, max_db,
+                                                        out.ctypes.data, out.nbytes))
+        return out
+
+    def spectrum_persistence_device(self, d_iq_ptr, iq_bytes, params, n_levels, min_db, max_db, d_counts, out_bytes,
+                                    stream=0):
+        """Device-resident variant (raw device pointers; d_counts holds n_levels * nfft uint32), asynchronous on
+        `stream`."""
+        _capi.check(_capi.lib().sa_spectrum_persistence_device(self._h, d_iq_ptr, iq_bytes, C.byref(params), n_levels,
+                                                               min_db, max_db, d_counts, out_bytes, stream))
+
     def iq_pack(self, iq, fmt):
         """IqData.getInterleavedBinary (IqData.java:160-187): bytes of interleaved LE float32 / int16."""
         if fmt.lower() not in _capi.PACK:
